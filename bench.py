@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- Msamples/s of the per-sample render loop (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2] [--dump-outputs DIR]
 
 A "step" is one Tracer::render call over one frame of the workload.  The metric is Msamples/s
 (GEODESIC): the default workload is the lensed one -- at N = 1 BASELINE configs[2] (C3: scene.json.gz +
@@ -13,6 +13,8 @@ the frame at C3's spp; `--workload C5` runs the full thing).  `--workload` picks
 C1-C4 are weak-scaled at N > 1 (every rank renders its own pass slice of the same frame size).
 Rank 0 prints ONE JSON line.  `--impl reference` times the reference algorithm's CPU restatement
 (oracle/, kind "port": the Rust crate cannot be built here) on a bounded sample of the same frame.
+`--dump-outputs DIR` writes the frame of the last timed step (see dump_outputs) so that two builds can be
+compared output for output: with the same arguments every run renders the same sample sets of the same scene.
 """
 import argparse
 import json
@@ -66,6 +68,26 @@ def make_config(name, world):
 
 def default_workload(world):
     return "C3" if world == 1 else "C5-64"
+
+
+DUMP_BYTES = 60_000_000      # the .npy headers stay within 64 MB as well
+
+
+def dump_outputs(out_dir, frame):
+    """Writes the RGBA32F frame a caller of the timed path receives (running sums, (h, w, 4)) as out_dir/frame.npy.
+    A frame above DUMP_BYTES is written as a fixed sample of its pixels instead: frame.npy (k, 4) holds the pixels
+    whose flat indices (y * w + x, ascending, float64) are in frame_pixels.npy; the sample depends only on the frame
+    size (seed 0), so runs with the same arguments write the same pixels."""
+    os.makedirs(out_dir, exist_ok=True)
+    frame = np.ascontiguousarray(frame, np.float32)
+    h, w, c = frame.shape
+    if frame.nbytes <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "frame.npy"), frame)
+        return
+    k = DUMP_BYTES // (c * 4 + 8)                   # values + a float64 index per sampled pixel
+    pixels = np.sort(np.random.default_rng(0).choice(h * w, k, replace=False))
+    np.save(os.path.join(out_dir, "frame.npy"), frame.reshape(h * w, c)[pixels])
+    np.save(os.path.join(out_dir, "frame_pixels.npy"), pixels.astype(np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -126,9 +148,9 @@ def cpu_sample(name, passes):
     cores = os.cpu_count() or 1
     cfg = O.make_config(samples=passes, subsample=sub)
     t0 = time.perf_counter()
-    _, n, _ = osc.render(cam, cfg, w, h, seed=0, n_threads=cores)
+    img, n, _ = osc.render(cam, cfg, w, h, seed=0, n_threads=cores)
     dt = time.perf_counter() - t0
-    return w * h * n / dt / 1e6, cores, n, dt, (w, h)
+    return w * h * n / dt / 1e6, cores, n, dt, (w, h), img
 
 
 def run_reference(args, json_out):
@@ -144,8 +166,10 @@ def run_reference(args, json_out):
         cpu_sample(name, passes)
     t = 0.0
     for _ in range(args.steps):
-        v, cores, n, dt, (sw, sh) = cpu_sample(name, passes)
+        v, cores, n, dt, (sw, sh), img = cpu_sample(name, passes)
         t += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, img)
     value = sw * sh * n * args.steps / t / 1e6
     sample = f"{n} spp of the frame at {sw}x{sh} per step (the full step is {d['spp']} spp at {d['width']}x{d['height']})"
     json_out.write(json.dumps({
@@ -215,6 +239,8 @@ def main():
     ap.add_argument("--workload", default=None, choices=sorted(WORKLOADS),
                     help="default: C3 on one GPU, C5-64 (the C5 frame at 64 spp, strong-scaled) on several")
     ap.add_argument("--no-extras", action="store_true", help="skip cpu_baseline / stepper roofline / other scenes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step to DIR/frame.npy (a fixed pixel sample above 60 MB)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args, json_out)
@@ -303,13 +329,15 @@ def main():
         ms, reduce_ms = float(t[0].item()), float(t[1].item())
     samples_per_step = w * h * d["spp"] * (1 if strong else n_gpus)
     value = samples_per_step * args.steps / (ms * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:     # before the e2e steps below reuse `frame`
+        dump_outputs(args.dump_outputs, frame.data.cpu().numpy())
 
     # ---- e2e: the same step with HOST buffers at N ranks -------------------------------------------
     # N = 1: the blocking C-ABI call with a pinned host frame (bt_render, BT_MEM_HOST: upload, kernels and download
     # inside the call, pipelined in row bands).  N > 1: rank 0 uploads the caller's pinned host frame (the running
     # sums), every rank renders its pass slice on its GPU, ONE NCCL reduce adds the slices onto rank 0's frame, rank 0
     # downloads it.  Wall clock between barriers around each step, max over ranks.
-    n_e2e = max(2, min(args.steps, 3))
+    n_e2e = args.steps
     host = dhost = None
     if rank == 0:
         host = torch.zeros((h, w, 4), dtype=torch.float32).pin_memory()
@@ -486,7 +514,7 @@ def main():
         result["scenes"] = scenes
     if rank == 0 and not args.no_extras:
         # ---- CPU baseline: the reference algorithm's restatement on this box's host cores (rank 0, bounded sample) ----
-        v, cores, n, dt, (sw, sh) = cpu_sample(name, 4 if not lens else 1)
+        v, cores, n, dt, (sw, sh), _ = cpu_sample(name, 4 if not lens else 1)
         result["cpu_baseline"] = {"value": v, "unit": METRIC, "cores": cores, "kind": "port",
                                   "sample": f"{n} spp of the frame at {sw}x{sh} ({dt:.1f} s wall on {cores} threads)"}
     if rank == 0:

@@ -74,15 +74,14 @@ UPSTREAM_DIR = os.path.join(ROOT, "tests", "golden", "scenes_upstream")
 
 @pytest.mark.parametrize("name", SCENES)
 def test_upstream_scene_bytes(name):
-    """the reference's shipped files, byte for byte (hash-ordered keys, the reference's own gzip stream): they load, round-trip
-    to the same JSON value, and flatten to exactly what the re-serialised copy flattens to"""
+    """the reference's shipped files, byte for byte (hash-ordered keys, the reference's own gzip stream; SHA256SUMS holds the
+    hashes of the reference's files): they load, round-trip to the same JSON value, and flatten to exactly what the
+    re-serialised copy flattens to"""
     import hashlib
     path = os.path.join(UPSTREAM_DIR, name + ".json.gz")
     sums = dict(reversed(l.split()) for l in open(os.path.join(UPSTREAM_DIR, "SHA256SUMS")))
     raw = open(path, "rb").read()
     assert hashlib.sha256(raw).hexdigest() == sums[name + ".json.gz"]
-    if os.path.exists(f"/root/reference/{name}.json.gz"):       # (not on the GPU box)
-        assert raw == open(f"/root/reference/{name}.json.gz", "rb").read()
     up, ours = bt.Scene(raw), bt.Scene.load(O.scene_path(name))
     original = json.loads(gzip.decompress(raw))
     assert list(original["objects"]["collection"]) != sorted(original["objects"]["collection"], key=int) or name != "cornell"
@@ -299,14 +298,15 @@ def test_cli_builtin_scene_and_flags(tmp_path):
     assert json.load(open(out))["objects"]["collection"]["0"]["inner"]["Camera"]["aspect_ratio"] == 1.5   # w / h
 
 
-def test_bench_reference_arm_contract():
+def test_bench_reference_arm_contract(tmp_path):
     """`bench.py --impl reference` (the reference algorithm on the host cores): one JSON line with the
-    contract's keys; under torchrun only rank 0 prints, the other ranks exit 0 without work."""
+    contract's keys; under torchrun only rank 0 prints, the other ranks exit 0 without work.  `--dump-outputs`
+    writes the frame of the last timed step: the oracle's image of that step."""
     import subprocess
     import sys
     root = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..")
     cmd = [sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
-           "--workload", "C1"]
+           "--workload", "C1", "--dump-outputs", str(tmp_path)]
     out = subprocess.run(cmd, capture_output=True, text=True, check=True, env={**os.environ, "RANK": "0"}).stdout
     lines = [l for l in out.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -316,8 +316,32 @@ def test_bench_reference_arm_contract():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": "Msamples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "C1" in d["config"]["workload"]
+    osc = O.OracleScene.load(O.scene_path("cornell"))
+    osc.set_camera_aspect(0, 1.0)
+    ref, _, _ = osc.render(0, O.make_config(samples=1, subsample=2), 512, 512, seed=0)
+    assert sorted(os.listdir(tmp_path)) == ["frame.npy"]
+    assert np.array_equal(np.load(tmp_path / "frame.npy"), ref)
+    os.remove(tmp_path / "frame.npy")
     other = subprocess.run(cmd, capture_output=True, text=True, check=True, env={**os.environ, "RANK": "1"})
-    assert other.stdout.strip() == ""
+    assert other.stdout.strip() == "" and os.listdir(tmp_path) == []
+
+
+def test_bench_dump_outputs_samples_large_frames(tmp_path, monkeypatch):
+    """a frame above bench.DUMP_BYTES is dumped as the same seeded pixel sample on every run, with its flat indices"""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * 24)
+    frame = np.random.default_rng(2).random((30, 40, 4), dtype=np.float32)
+    for run in ("a", "b"):
+        bench.dump_outputs(tmp_path / run, frame)
+        assert sorted(os.listdir(tmp_path / run)) == ["frame.npy", "frame_pixels.npy"]
+    values, pixels = np.load(tmp_path / "a" / "frame.npy"), np.load(tmp_path / "a" / "frame_pixels.npy")
+    assert values.shape == (100, 4) and values.dtype == np.float32 and pixels.dtype == np.float64
+    assert (np.diff(pixels) > 0).all() and pixels[-1] < 30 * 40
+    assert np.array_equal(values, frame.reshape(-1, 4)[pixels.astype(np.int64)])
+    assert np.array_equal(np.load(tmp_path / "b" / "frame_pixels.npy"), pixels)
+    assert np.array_equal(np.load(tmp_path / "b" / "frame.npy"), values)
+    bench.dump_outputs(tmp_path / "small", frame[:5, :5])
+    assert np.array_equal(np.load(tmp_path / "small" / "frame.npy"), frame[:5, :5])
 
 
 def test_rust_sys_crate_matches_header():
@@ -380,16 +404,31 @@ def test_reference_patch_is_well_formed():
     for struct in ("bt_config", "bt_render_config"):
         body = re.search(r"sys::%s \{(.*?)\n        \};" % struct, added, flags=re.S).group(1)
         assert re.findall(r"^ {12}(\w+):", body, flags=re.M) == [f for f, _, _ in structs[struct]], struct
-    if os.path.isdir("/root/reference/src"):      # (not on the GPU box) the patch applies to the reference as it is
-        import shutil
-        import subprocess
-        import tempfile
-        with tempfile.TemporaryDirectory() as tmp:
-            shutil.copytree("/root/reference/src", os.path.join(tmp, "src"))
-            shutil.copy("/root/reference/Cargo.toml", tmp)
-            r = subprocess.run(["patch", "-p1", "--dry-run", "-i", os.path.join(ROOT, "patches", "bendy_tracer_b200.patch")],
-                               cwd=tmp, capture_output=True, text=True)
-            assert r.returncode == 0, r.stdout + r.stderr
+    # the hunks are consistent on their own (what `patch -p1` checks before it reads the reference's files; inside a
+    # checkout of the reference, `patch -p1 --dry-run -i patches/bendy_tracer_b200.patch` checks the rest): every body
+    # has the line counts of its header, and a file's hunks are in order, disjoint, and start where the net growth of
+    # the hunks before them puts them
+    lines = patch.splitlines()
+    i = n_hunks = 0
+    while i < len(lines):
+        if lines[i].startswith("--- "):
+            assert lines[i + 1].startswith("+++ "), lines[i]
+            i, old_end, growth = i + 2, 0, 0
+            continue
+        m = re.fullmatch(r"@@ -(\d+)(?:,(\d+))? \+(\d+)(?:,(\d+))? @@.*", lines[i])
+        assert m, f"line {i + 1}: {lines[i]!r}"
+        old_start, n_old, new_start, n_new = (int(g) if g is not None else 1 for g in m.groups())
+        assert old_start > old_end and new_start == old_start + growth, lines[i]
+        old_end, growth, n_hunks = old_start + n_old - 1, growth + n_new - n_old, n_hunks + 1
+        i += 1
+        while n_old or n_new:
+            tag = lines[i][:1] if i < len(lines) else "end of file"
+            assert tag in (" ", "-", "+") and (n_old > 0 or tag == "+") and (n_new > 0 or tag == "-"), \
+                f"line {i + 1}: the hunk body does not match its header"
+            n_old -= tag != "+"
+            n_new -= tag != "-"
+            i += 1
+    assert n_hunks == 7
 
 
 def test_json_nesting_limit_is_an_error_not_a_crash():
