@@ -63,6 +63,7 @@ SIGNATURES = {
     "bt_scene_commit": (C.c_int, [_P]),
     "bt_scene_set_lenses": (C.c_int, [_P, _P, C.c_uint32, C.POINTER(BtLensConfig)]),
     "bt_lens_config_default": (None, [C.POINTER(BtLensConfig)]),
+    "bt_scene_set_environment": (C.c_int, [_P, _P, C.c_uint32, C.c_uint32]),
     "bt_scene_set_accel": (C.c_int, [_P, C.c_int]),
     "bt_scene_set_precision": (C.c_int, [_P, C.c_int]),
     "bt_scene_get_info": (C.c_int, [_P, C.POINTER(BtSceneInfo)]),

@@ -266,6 +266,20 @@ class Scene:
         cfg = (lens_config or LensConfig())._c()
         check(lib.bt_scene_set_lenses(self.handle, xyzr.ctypes.data, len(xyzr), C.byref(cfg)))
 
+    def set_environment(self, rgb):
+        """environment map (bt_scene_set_environment): an equirectangular (H, W, 3) RGB image that multiplies the colour of
+        every escaping path, looked up in its escape direction; row 0 is the +y pole, the centre column looks along -z.
+        None clears it.  Negative or non-finite values raise BendyError (BT_ERR_INVALID_ARG), a wrong shape ValueError."""
+        if rgb is None:
+            check(lib.bt_scene_set_environment(self.handle, None, 0, 0))
+            return
+        rgb = np.ascontiguousarray(rgb, np.float32)
+        if rgb.ndim != 3 or rgb.shape[2] != 3 or rgb.shape[0] == 0 or rgb.shape[1] == 0:
+            raise ValueError(f"environment map must be a non-empty (H, W, 3) array, got shape {rgb.shape}")
+        if rgb.shape[0] * rgb.shape[1] >= 1 << 31:
+            raise ValueError(f"environment map of {rgb.shape[0]} x {rgb.shape[1]} texels: width * height must be below 2^31")
+        check(lib.bt_scene_set_environment(self.handle, rgb.ctypes.data, rgb.shape[1], rgb.shape[0]))
+
     def set_accel(self, accel):
         """closest-hit structure: "auto" (linear scan up to 64 primitives, BVH beyond), "linear", "bvh",
         "linear_faces" (the scan with every cuboid as six rect tests, no box slab test)"""

@@ -3,7 +3,7 @@
 //
 //   bendy_b200_cli --output full|albedo|normal [--width 768] [--height 512] [--samples 64]
 //                  [--subsample 2] [--screenshot screenshots/render.png] [--scene scene.json]
-//                  [--lens x,y,z,r_s] [--seed 0] [--save-scene out.json(.gz)]
+//                  [--lens x,y,z,r_s] [--environment sky.pfm] [--seed 0] [--save-scene out.json(.gz)]
 //
 // Same flags, defaults and semantics as the reference's clap CLI: `--output` is required; the scene
 // file is read when it exists (gzip when the extension is .gz), otherwise the built-in Cornell box
@@ -11,9 +11,12 @@
 // (main.rs:216-223); the tracer runs ONE pass per iteration (`samples = 1`) until
 // buffer.samples() >= --samples (main.rs:248-254; buffer.samples() counts sub-samples); the preview
 // is written as PNG (what Ctrl+P does, main.rs:275-298).  Instead of the title bar the per-pass
-// time, average and total are printed to stderr (main.rs:352-388).
+// time, average and total are printed to stderr (main.rs:352-388).  --environment (an extension, like --lens) sets an
+// equirectangular environment map from a PFM file (bt_scene_set_environment); a malformed file is an error even in the
+// GPU-less --samples 0 dry run.
 #include <zlib.h>
 
+#include <cctype>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -144,13 +147,61 @@ bool write_png(const std::string& path, const std::vector<uint8_t>& rgba, uint32
     return (bool)f;
 }
 
+// ---- PFM (the float image format: "PF" RGB / "Pf" grey, then "W H", then scale -- negative: little-endian --, one
+// whitespace byte and W * H pixels of 32-bit floats, bottom row first) -> top-row-first RGB -------------------
+std::vector<float> read_pfm(const std::string& path, uint32_t* w_out, uint32_t* h_out) {
+    std::ifstream in(path, std::ios::binary);
+    if (!in) die("cannot open environment map " + path);
+    std::string bytes((std::istreambuf_iterator<char>(in)), std::istreambuf_iterator<char>());
+    size_t at = 0;
+    auto token = [&]() -> std::string {
+        while (at < bytes.size() && std::isspace((unsigned char)bytes[at])) ++at;
+        const size_t start = at;
+        while (at < bytes.size() && !std::isspace((unsigned char)bytes[at])) ++at;
+        return bytes.substr(start, at - start);
+    };
+    const std::string magic = token(), ws = token(), hs = token(), ss = token();
+    if (magic != "PF" && magic != "Pf") die(path + ": not a PFM file (header must start with PF or Pf)");
+    char* end = nullptr;
+    const unsigned long long w = std::strtoull(ws.c_str(), &end, 10);
+    if (ws.empty() || *end || ws[0] == '-' || w == 0) die(path + ": bad PFM width '" + ws + "'");
+    const unsigned long long h = std::strtoull(hs.c_str(), &end, 10);
+    if (hs.empty() || *end || hs[0] == '-' || h == 0) die(path + ": bad PFM height '" + hs + "'");
+    const double scale = std::strtod(ss.c_str(), &end);
+    if (ss.empty() || *end || !(scale != 0.0) || !std::isfinite(scale)) die(path + ": bad PFM scale '" + ss + "'");
+    if (at >= bytes.size() || !std::isspace((unsigned char)bytes[at])) die(path + ": truncated PFM header");
+    ++at;  // the single whitespace byte that ends the header
+    if (w >= (1ull << 31) || h >= (1ull << 31) || w * h >= (1ull << 31)) die(path + ": PFM image too large");
+    const size_t ch = magic == "PF" ? 3 : 1, n = (size_t)(w * h) * ch;
+    if (bytes.size() - at < n * 4)
+        die(path + ": truncated PFM data (" + std::to_string(bytes.size() - at) + " bytes, " + std::to_string(n * 4) + " expected)");
+    const bool little = scale < 0.0;
+    const uint16_t probe = 1;
+    const bool host_little = *(const unsigned char*)&probe == 1;
+    std::vector<float> rgb((size_t)(w * h) * 3);
+    for (size_t y = 0; y < h; ++y)
+        for (size_t x = 0; x < w; ++x)
+            for (size_t c = 0; c < 3; ++c) {
+                unsigned char b[4];
+                std::memcpy(b, bytes.data() + at + (((h - 1 - y) * w + x) * ch + (ch == 3 ? c : 0)) * 4, 4);
+                if (little != host_little) {
+                    std::swap(b[0], b[3]);
+                    std::swap(b[1], b[2]);
+                }
+                std::memcpy(&rgb[(y * w + x) * 3 + c], b, 4);
+            }
+    *w_out = (uint32_t)w;
+    *h_out = (uint32_t)h;
+    return rgb;
+}
+
 }  // namespace
 
 int main(int argc, char** argv) {
     uint32_t width = 768, height = 512, subsample = 2;
     uint64_t samples = 64, seed = 0;
     int output = -1;
-    std::string screenshot = "screenshots/render.png", scene_path = "scene.json", save_scene;
+    std::string screenshot = "screenshots/render.png", scene_path = "scene.json", save_scene, environment;
     std::vector<float> lens;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
@@ -166,6 +217,7 @@ int main(int argc, char** argv) {
         else if (a == "--screenshot") screenshot = val();
         else if (a == "--scene") scene_path = val();
         else if (a == "--save-scene") save_scene = val();
+        else if (a == "--environment") environment = val();
         else if (a == "--lens") {
             std::stringstream ss(val());
             std::string tok;
@@ -194,6 +246,12 @@ int main(int argc, char** argv) {
         ck(bt_scene_create_json(engine, text.data(), text.size(), &scene), "built-in scene");
     }
     if (!lens.empty()) ck(bt_scene_set_lenses(scene, lens.data(), (uint32_t)(lens.size() / 4), nullptr), "lenses");
+    if (!environment.empty()) {
+        uint32_t ew = 0, eh = 0;
+        const std::vector<float> rgb = read_pfm(environment, &ew, &eh);
+        ck(bt_scene_set_environment(scene, rgb.data(), ew, eh), ("environment map " + environment).c_str());
+        std::fprintf(stderr, "environment map %s: %u x %u\n", environment.c_str(), ew, eh);
+    }
     uint64_t camera = 0;
     ck(bt_scene_find_by_tag(scene, "camera", &camera), "find_by_tag(\"camera\")");
     ck(bt_scene_set_camera_aspect(scene, camera, (float)width / (float)height), "camera aspect");  // main.rs:218-223

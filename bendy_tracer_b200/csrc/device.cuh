@@ -883,6 +883,31 @@ BT_DEV float density_trilinear(const float4* vol, const float* grids, V3 coord) 
 }
 
 // ------------------------------------------------------------------------------------------
+// environment map (extension, DESIGN.md "Environment map"): the factor sample_root's colour is multiplied by
+// ------------------------------------------------------------------------------------------
+// Equirectangular texels (float4, .w unused: one LDG.128 per tap), row 0 = the +y pole, the centre column looks
+// along -z, columns grow towards +x.  Bilinear; columns wrap, rows clamp.  The test oracle's lookup (tests/oracle_env.cpp) is the same
+// operation sequence: every product and sum is rounded on its own (x*_rn intrinsics), so no FMA contraction -- which
+// the fast flavour would decide per kernel -- can make the pooled and the lane kernel disagree; the flavours differ
+// only in m_sqrt.  x and y are clamped to [-1, W] / [-1, H] before any index is formed (fmaxf returns the non-NaN
+// operand, so a NaN lands on -1): no direction -- zero, non-unit, NaN or infinite components -- reads outside the map,
+// and the weights are always finite, so a constant map returns its constant exactly (a + (b - a) t = a).
+BT_DEV float xlerp(float a, float b, float t) { return __fadd_rn(a, __fmul_rn(__fsub_rn(b, a), t)); }
+BT_DEV V3 env_lookup(const float4* env, uint32_t w, uint32_t h, V3 d) {
+    const float phi = atan2f(d.x, -d.z), theta = atan2f(d.y, m_sqrt(__fadd_rn(__fmul_rn(d.x, d.x), __fmul_rn(d.z, d.z))));
+    const float u = __fadd_rn(0.5f, __fmul_rn(phi, 0.159154943091895335769f)), v = __fsub_rn(0.5f, __fmul_rn(theta, 0.318309886183790671538f));
+    const float x = fminf(fmaxf(__fsub_rn(__fmul_rn(u, (float)w), 0.5f), -1.0f), (float)w);
+    const float y = fminf(fmaxf(__fsub_rn(__fmul_rn(v, (float)h), 0.5f), -1.0f), (float)h);
+    const float fx = floorf(x), fy = floorf(y), tx = __fsub_rn(x, fx), ty = __fsub_rn(y, fy);
+    const uint32_t c0 = fx < 0.0f ? w - 1 : min((uint32_t)fx, w - 1), c1 = c0 + 1 == w ? 0 : c0 + 1;
+    const uint32_t r0 = fy < 0.0f ? 0 : min((uint32_t)fy, h - 1), r1 = fy < 0.0f ? 0 : min((uint32_t)fy + 1, h - 1);
+    const float4 a = __ldg(env + r0 * w + c0), b = __ldg(env + r0 * w + c1), c = __ldg(env + r1 * w + c0), e = __ldg(env + r1 * w + c1);
+    const V3 top = v3(xlerp(a.x, b.x, tx), xlerp(a.y, b.y, tx), xlerp(a.z, b.z, tx));
+    const V3 bot = v3(xlerp(c.x, e.x, tx), xlerp(c.y, e.y, tx), xlerp(c.z, e.z, tx));
+    return v3(xlerp(top.x, bot.x, ty), xlerp(top.y, bot.y, ty), xlerp(top.z, bot.z, ty));
+}
+
+// ------------------------------------------------------------------------------------------
 // camera (mod.rs:272-302, ray.rs:103-137)
 // ------------------------------------------------------------------------------------------
 BT_DEV V3 with_frustum_dir(float yfov, float xfov, float u, float v) {

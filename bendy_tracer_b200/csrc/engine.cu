@@ -101,6 +101,9 @@ struct SceneDev {
     size_t grids_cap;
     uint8_t* d_dist;    // free-distance grid (FlatScene::dist)
     size_t dist_cap;
+    uint64_t env_version;  // bt_scene::env_version this copy's environment map holds
+    float4* d_env;
+    size_t env_cap;
 };
 
 struct bt_scene {
@@ -119,6 +122,11 @@ struct bt_scene {
     std::vector<std::pair<uint32_t, uint32_t> > patch;
     uint64_t patch_base;
     bool patch_dist;    // ... and the free-distance grid too
+    // environment map (bt_scene_set_environment): env_w x env_h float4 texels (.w = 0), uploaded on its own -- setting or
+    // clearing it never re-flattens the scene.  env_version is bumped by every set / clear (0: never set).
+    std::vector<float4> env;
+    uint32_t env_w, env_h;
+    uint64_t env_version;
     std::vector<SceneDev> devs;
 };
 
@@ -289,6 +297,24 @@ int refresh_scene(bt_scene* s, int device, cudaStream_t stream, SceneDev** out) 
         CK(cudaStreamSynchronize(stream));  // the host vectors may change after we return
         d->version = s->flat_version;
     }
+    if (d->env_version != s->env_version) {
+        // the environment map on its own (the flattened scene does not depend on it); a render enqueued without
+        // synchronising may still be reading the old texels
+        if (d->ev_use) CK(cudaEventSynchronize(d->ev_use));
+        const size_t eb = s->env.size() * sizeof(float4);
+        if (eb > d->env_cap) {
+            if (d->d_env) cudaFree(d->d_env);
+            d->d_env = 0;
+            d->env_cap = 0;
+            CK(cudaMalloc((void**)&d->d_env, eb));
+            d->env_cap = eb;
+        }
+        if (eb) {
+            CK(cudaMemcpyAsync(d->d_env, s->env.data(), eb, cudaMemcpyHostToDevice, stream));
+            CK(cudaStreamSynchronize(stream));
+        }
+        d->env_version = s->env_version;
+    }
     *out = d;
     return BT_OK;
 }
@@ -333,6 +359,9 @@ int build_params(const bt_engine* en, bt_scene* s, const SceneDev* dev, uint64_t
     p.blob = dev->d_blob;
     p.grids = dev->d_grids;
     p.dist = dev->d_dist;
+    p.env = dev->d_env;
+    p.env_w = s->env.empty() ? 0u : s->env_w;
+    p.env_h = s->env_h;
     p.width = width;
     p.height = height;
     if (m.samples * p.sub_count > 0xffffffffULL) return fail(BT_ERR_INVALID_ARG, "samples * subpixel_count exceeds 2^32 per call");
@@ -607,6 +636,7 @@ void bt_scene_destroy(bt_scene* scene) {
         if (d.d_blob) cudaFree(d.d_blob);
         if (d.d_grids) cudaFree(d.d_grids);
         if (d.d_dist) cudaFree(d.d_dist);
+        if (d.d_env) cudaFree(d.d_env);
     }
     delete scene;
 }
@@ -683,6 +713,32 @@ int bt_scene_set_lenses(bt_scene* scene, const float* xyzr, uint32_t n, const bt
     scene->scene.lens_config.flags = c.flags;
     scene->flat_dirty = true;
     return BT_OK;
+}
+
+int bt_scene_set_environment(bt_scene* scene, const float* rgb, uint32_t width, uint32_t height) {
+    if (!scene) return fail(BT_ERR_INVALID_ARG, "NULL argument");
+    if (!rgb) {
+        if (width != 0 || height != 0) return fail(BT_ERR_INVALID_ARG, "environment map: NULL texels need width = height = 0 (clear)");
+        std::vector<float4>().swap(scene->env);
+        scene->env_w = scene->env_h = 0;
+        ++scene->env_version;
+        return BT_OK;
+    }
+    if (width == 0 || height == 0) return fail(BT_ERR_INVALID_ARG, "environment map: width and height must be positive");
+    if ((uint64_t)width * height >= (1ull << 31)) return fail(BT_ERR_INVALID_ARG, "environment map: width * height must be below 2^31");
+    const size_t n = (size_t)width * height;
+    for (size_t i = 0; i < 3 * n; ++i)
+        if (!(rgb[i] >= 0.0f && rgb[i] <= 3.402823466e38f))
+            return fail(BT_ERR_INVALID_ARG, "environment map: texel " + std::to_string(i / 3) + " is negative or not finite");
+    GUARD_BEGIN
+    std::vector<float4> texels(n);
+    for (size_t i = 0; i < n; ++i) texels[i] = make_float4(rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2], 0.0f);
+    scene->env.swap(texels);
+    scene->env_w = width;
+    scene->env_h = height;
+    ++scene->env_version;
+    return BT_OK;
+    GUARD_END
 }
 
 int bt_scene_set_accel(bt_scene* scene, int accel) {

@@ -328,8 +328,9 @@ BT_DEV bool shade_event(const RenderParams& p, const SceneView& sc, const Consts
     // ---- 1. classify the event ----------------------------------------------------------------
     if (tr.h.prim < 0) {
         finish = true;
-        if (!tr.captured) {  // sample_root, mod.rs:429-452
+        if (!tr.captured) {  // sample_root, mod.rs:429-452 (times the environment map in the escape direction)
             fin_color = v3(p.scene.root_color[0], p.scene.root_color[1], p.scene.root_color[2]);
+            if (p.env_w != 0) fin_color = fin_color * env_lookup(p.env, p.env_w, p.env_h, tr.d);
             fin_albedo = v3(p.scene.root_albedo[0], p.scene.root_albedo[1], p.scene.root_albedo[2]);
             if (p.scene.root_keeps_normal) {
                 fin_normal = -tr.d;

@@ -126,6 +126,8 @@ struct RenderParams {
     const float4* blob;
     const float* grids;
     const uint8_t* dist;             // the free-distance grid (SceneHeader::dist_*), device memory
+    const float4* env;               // environment map (bt_scene_set_environment): env_w x env_h texels, .w unused, device memory
+    uint32_t env_w, env_h;           // env_w == 0: no map
     float4* fb;
     uint32_t width, height;
     uint32_t paths_per_pixel;        // samples * subpixel_count of this call

@@ -163,6 +163,18 @@ int bt_scene_commit(bt_scene* scene);
 /* lens field: n point masses (x, y, z, r_s); cfg may be NULL for the defaults */
 int bt_scene_set_lenses(bt_scene* scene, const float* xyzr, uint32_t n, const bt_lens_config* cfg);
 void bt_lens_config_default(bt_lens_config* cfg);
+/* Environment map (extension; DESIGN.md "Environment map"): an equirectangular RGB image the colour of every escaping
+ * path is multiplied by, looked up in its escape direction d (the straight ray, the last chord / final velocity of a
+ * bent flight, the march direction of a volume escape): colour = sample_root's colour * env(d).  Albedo, normal and
+ * depth outputs, captured flights, paths and RNG draws are unchanged; with the root Emissive{white, k} the sky shows
+ * k * map, with a Flat{black} root nothing.  rgb = width * height * 3 floats in host memory, row-major: row 0 is the +y
+ * pole, row height-1 the -y pole, the centre column looks along -z (the default camera's view) and columns grow
+ * towards +x.  Lookup: phi = atan2(d.x, -d.z), theta = atan2(d.y, sqrt(d.x^2 + d.z^2)), u = 0.5 + phi / 2pi,
+ * v = 0.5 - theta / pi, texel coordinates (u W - 0.5, v H - 0.5), bilinear, columns wrap, rows clamp.  The texels are
+ * copied (the caller may free rgb); rgb = NULL with width = height = 0 clears the map.  BT_ERR_INVALID_ARG (scene
+ * unchanged) for zero or inconsistent sizes, width * height >= 2^31, negative or non-finite values.  Like the lens
+ * field it is not part of the wire format (bt_scene_to_json is unchanged), and setting it never re-flattens the scene. */
+int bt_scene_set_environment(bt_scene* scene, const float* rgb, uint32_t width, uint32_t height);
 /* Closest-hit structure.  AUTO: the reference's linear scan (try_hit, src/tracer/mod.rs:389-402)
  * over shared memory up to 64 flattened primitives, a BVH (global-memory nodes, shared-memory
  * traversal stack) beyond.  Both give the same hits, exact-distance ties included.  Scenes with
