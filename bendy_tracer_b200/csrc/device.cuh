@@ -995,26 +995,46 @@ BT_DEV float rsqrt_approx(float x) {
     asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
+// The stepper's vectors as one register pair (x, y) and a single z: the x and y components of every vector operation
+// go through one paired FP32 instruction (FFMA2 / FADD2 / FMUL2, sm_100), z through a scalar one.  Each component is
+// the operation the scalar code would perform, correctly rounded on its own (the paired intrinsics round per component
+// like __fmaf_rn / __fadd_rn / __fmul_rn), so the pairing changes no bit.  The pairs cost no MOV as long as the
+// pair of a value stays the same pair: the stepper, the chord and the pooled STEP loop all keep this one layout.
+struct P3 {
+    float2 xy;
+    float z;
+};
+BT_DEV P3 p3(float2 xy, float z) { P3 r = {xy, z}; return r; }
+BT_DEV P3 p3(V3 a) { return p3(make_float2(a.x, a.y), a.z); }
+BT_DEV P3 p3(float4 q) { return p3(make_float2(q.x, q.y), q.z); }
+BT_DEV V3 v3(P3 a) { return v3(a.xy.x, a.xy.y, a.z); }
+BT_DEV float2 f2(float a) { return make_float2(a, a); }
+BT_DEV P3 operator+(P3 a, P3 b) { return p3(__fadd2_rn(a.xy, b.xy), __fadd_rn(a.z, b.z)); }
+// a - b as a + (-b): the same IEEE operation (a FADD2 with a negated operand)
+BT_DEV P3 operator-(P3 a, P3 b) { return p3(__fadd2_rn(a.xy, make_float2(-b.xy.x, -b.xy.y)), __fsub_rn(a.z, b.z)); }
+BT_DEV P3 axpy(float a, P3 x, P3 y) { return p3(__ffma2_rn(f2(a), x.xy, y.xy), __fmaf_rn(a, x.z, y.z)); }
 // Per-step cache of d0_m = x - c_m, filled by the k1 evaluation and reused by the three stage
 // evaluations (register-resident tables only; the shared-memory walk recomputes it).
 template <class L>
 struct D0Cache {
     enum { CACHED = 0 };
-    BT_DEV V3 get(int, V3 x, float4 e0) const { return v3(x.x - e0.x, x.y - e0.y, x.z - e0.z); }
-    BT_DEV void put(int, V3) {}
+    BT_DEV P3 get(int, P3 x, float4 e0) const { return x - p3(e0); }
+    BT_DEV void put(int, P3) {}
 };
 template <int N>
 struct D0Cache<LensRegs<N> > {
     enum { CACHED = 1 };
-    V3 d[N];
-    BT_DEV V3 get(int m, V3, float4) const { return d[m]; }
-    BT_DEV void put(int m, V3 v) { d[m] = v; }
+    P3 d[N];
+    BT_DEV P3 get(int m, P3, float4) const { return d[m]; }
+    BT_DEV void put(int m, P3 v) { d[m] = v; }
 };
 // a = sum_m -(3/2) r_s |d x v|^2 d / |d|^5 evaluated at x + a*w, written as d = fma(a, w, x - c)
 // (STAGE 0: a = 0, d = x - c).  INFO 1 also returns min |d|; INFO 2 adds the capture / far flags.
+// d, w, v and the sum are paired (P3); |d|^2, the cross product and what follows from it stay scalar: each is a chain
+// whose x and y terms feed one another, or needs pairs such as (y, z) that the layout does not hold.
 template <int INFO, bool EXACT, int STAGE, class L>
-BT_DEV V3 lens_accel(const L& lens, D0Cache<L>& cache, V3 x, float a, V3 w, V3 v, float& rmin, bool& captured, bool& far) {
-    float ax = 0.0f, ay = 0.0f, az = 0.0f;
+BT_DEV P3 lens_accel(const L& lens, D0Cache<L>& cache, P3 x, float a, P3 w, P3 v, float& rmin, bool& captured, bool& far) {
+    P3 acc = p3(make_float2(0.0f, 0.0f), 0.0f);
     if (INFO >= 1) rmin = __int_as_float(0x7f800000);
     if (INFO >= 2) {
         captured = false;
@@ -1024,31 +1044,25 @@ BT_DEV V3 lens_accel(const L& lens, D0Cache<L>& cache, V3 x, float a, V3 w, V3 v
 #pragma unroll(L::UNROLL)
     for (int m = 0; m < n_lens; ++m) {
         const float4 e0 = lens.e0(m);  // (c.xyz, -1.5 r_s)
-        float dx, dy, dz;
+        P3 d;
         if (STAGE == 0) {
-            dx = x.x - e0.x;
-            dy = x.y - e0.y;
-            dz = x.z - e0.z;
-            cache.put(m, v3(dx, dy, dz));
+            d = x - p3(e0);
+            cache.put(m, d);
         } else {
-            const V3 d0 = cache.get(m, x, e0);
-            dx = fmaf(a, w.x, d0.x);
-            dy = fmaf(a, w.y, d0.y);
-            dz = fmaf(a, w.z, d0.z);
+            d = axpy(a, w, cache.get(m, x, e0));
         }
+        const float dx = d.xy.x, dy = d.xy.y, dz = d.z, vx = v.xy.x, vy = v.xy.y, vz = v.z;
         float r2 = fmaf(dz, dz, fmaf(dy, dy, dx * dx));
-        float lx = fmaf(dy, v.z, -(dz * v.y));
-        float ly = fmaf(dz, v.x, -(dx * v.z));
-        float lz = fmaf(dx, v.y, -(dy * v.x));
+        float lx = fmaf(dy, vz, -(dz * vy));
+        float ly = fmaf(dz, vx, -(dx * vz));
+        float lz = fmaf(dx, vy, -(dy * vx));
         float h2 = fmaf(lz, lz, fmaf(ly, ly, lx * lx));
         // fast: MUFU.RSQ (<= 2 ulp); exact: correctly rounded, bit-identical to the CPU oracle
         float inv = EXACT ? __frsqrt_rn(r2) : rsqrt_approx(r2);
         float inv2 = inv * inv;
         float inv5 = (inv2 * inv2) * inv;
         float s = (e0.w * h2) * inv5;
-        ax = fmaf(s, dx, ax);
-        ay = fmaf(s, dy, ay);
-        az = fmaf(s, dz, az);
+        acc = axpy(s, d, acc);
         if (INFO >= 1) {
             float r = r2 * inv;
             rmin = fminf(rmin, r);
@@ -1056,7 +1070,7 @@ BT_DEV V3 lens_accel(const L& lens, D0Cache<L>& cache, V3 x, float a, V3 w, V3 v
                 const float4 e1 = lens.e1(m);  // (r_s, r_far * r_s, -, -)
                 if (r < e1.x) captured = true;
                 if (r > e1.y) {  // beyond r_far of this mass (rare): receding?
-                    const float dv = fmaf(dz, v.z, fmaf(dy, v.y, dx * v.x));
+                    const float dv = fmaf(dz, vz, fmaf(dy, vy, dx * vx));
                     if (!(dv > 0.0f)) far = false;
                 } else {
                     far = false;
@@ -1064,23 +1078,22 @@ BT_DEV V3 lens_accel(const L& lens, D0Cache<L>& cache, V3 x, float a, V3 w, V3 v
             }
         }
     }
-    return v3(ax, ay, az);
+    return acc;
 }
-BT_DEV V3 axpy(float a, V3 x, V3 y) { return v3(fmaf(a, x.x, y.x), fmaf(a, x.y, y.y), fmaf(a, x.z, y.z)); }
 // classic RK4 given k1 = accel(x, v) (whose evaluation filled `cache`)
 template <bool EXACT, class L>
-BT_DEV void rk4_from_k1(const L& lens, D0Cache<L>& cache, V3& x, V3& v, V3 k1, float h) {
+BT_DEV void rk4_from_k1(const L& lens, D0Cache<L>& cache, P3& x, P3& v, P3 k1, float h) {
     float hh = 0.5f * h, h6 = h * (float)(1.0 / 6.0);
     float ru;
     bool bu;
-    V3 v2 = axpy(hh, k1, v);
-    V3 k2 = lens_accel<0, EXACT, 1>(lens, cache, x, hh, v, v2, ru, bu, bu);
-    V3 v3_ = axpy(hh, k2, v);
-    V3 k3 = lens_accel<0, EXACT, 1>(lens, cache, x, hh, v2, v3_, ru, bu, bu);
-    V3 v4 = axpy(h, k3, v);
-    V3 k4 = lens_accel<0, EXACT, 1>(lens, cache, x, h, v3_, v4, ru, bu, bu);
-    V3 sv = axpy(2.0f, v2 + v3_, v + v4);
-    V3 sk = axpy(2.0f, k2 + k3, k1 + k4);
+    P3 v2 = axpy(hh, k1, v);
+    P3 k2 = lens_accel<0, EXACT, 1>(lens, cache, x, hh, v, v2, ru, bu, bu);
+    P3 v3_ = axpy(hh, k2, v);
+    P3 k3 = lens_accel<0, EXACT, 1>(lens, cache, x, hh, v2, v3_, ru, bu, bu);
+    P3 v4 = axpy(h, k3, v);
+    P3 k4 = lens_accel<0, EXACT, 1>(lens, cache, x, h, v3_, v4, ru, bu, bu);
+    P3 sv = axpy(2.0f, v2 + v3_, v + v4);
+    P3 sk = axpy(2.0f, k2 + k3, k1 + k4);
     x = axpy(h6, sv, x);
     v = axpy(h6, sk, v);
 }
@@ -1088,11 +1101,12 @@ BT_DEV float step_size(float kappa, float h_min, float h_max, float rmin) { retu
 // chord direction and length.  EXACT: IEEE square root and reciprocal (the oracle's values);
 // otherwise one MUFU.RSQ (<= 2 ulp), like the stepper's own 1/|d|.
 template <bool EXACT>
-BT_DEV V3 normalize_fma(V3 a, float* len_out) {
-    float l2 = fmaf(a.z, a.z, fmaf(a.y, a.y, a.x * a.x));
+BT_DEV V3 normalize_fma(P3 a, float* len_out) {
+    const float ax = a.xy.x, ay = a.xy.y;
+    float l2 = fmaf(a.z, a.z, fmaf(ay, ay, ax * ax));
     float inv = EXACT ? 1.0f / sqrtf(l2) : rsqrt_approx(l2);
     if (len_out) *len_out = l2 * inv;
-    return a * inv;
+    return v3(ax * inv, ay * inv, a.z * inv);
 }
 
 }  // namespace bt

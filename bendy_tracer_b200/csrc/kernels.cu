@@ -80,7 +80,8 @@ BT_DEV Traced trace_straight(const RenderParams& p, const SceneView& sc, V3 o, V
     return r;
 }
 
-// A geodesic in flight: the state a lane carries between steps (x, v live in the caller's o, d).
+// A geodesic in flight: the state a lane carries between steps (x, v live in the caller's registers; they and xp are
+// held in the stepper's paired layout, P3).
 // Nothing else is written inside the flight loop: the event a resolved flight hands to shading is
 // rebuilt from this state afterwards (flight_result), which keeps the loop free of merge copies.
 struct Flight {
@@ -89,7 +90,7 @@ struct Flight {
     float free;  // no primitive surface lies within this distance of x (<= 0: unknown)
     float rest;  // the same for every primitive but `near`, whose distance is re-evaluated at each step
     int near;    // the sphere that bounded `free` at the last intersection pass (-1: none / not a sphere)
-    V3 xp;       // start of the last chord xp -> x that needed / needs an intersection test
+    P3 xp;       // start of the last chord xp -> x that needed / needs an intersection test
     Hit h;       // FL_HIT / FL_HIT_FAR: the hit on that chord (t relative to its start)
 };
 // Lane states.  In flight: FL_FLY ready for the next RK4 step; FL_PEND the step is taken (x, v
@@ -105,7 +106,7 @@ BT_DEV void flight_reset(Flight& f) {
     f.steps = f.scans = 0;
     f.free = f.rest = 0.0f;
     f.near = -1;
-    f.xp = v3(0.0f, 0.0f, 0.0f);
+    f.xp = p3(make_float2(0.0f, 0.0f), 0.0f);
     f.h.t = 0.0f;
     f.h.prim = -1;
     f.h.face = 0;
@@ -118,11 +119,13 @@ struct GridFetch {
     uint32_t raw;   // the cell's byte (inside the box)
     float other;    // min(outside-the-box bound or +inf, the scene-spanning spheres' exact bounds)
 };
-BT_DEV GridFetch grid_bound_fetch(const RenderParams& p, const float4* prims, V3 x) {
+BT_DEV GridFetch grid_bound_fetch(const RenderParams& p, const float4* prims, P3 px) {
     const SceneHeader& s = p.scene;
     // cell index: a negative coordinate converts to a negative int, i.e. a huge unsigned one
-    const uint32_t ix = (uint32_t)__float2int_rd((x.x - s.dist_lo[0]) * s.dist_inv_cell), iy = (uint32_t)__float2int_rd((x.y - s.dist_lo[1]) * s.dist_inv_cell),
-                   iz = (uint32_t)__float2int_rd((x.z - s.dist_lo[2]) * s.dist_inv_cell);
+    const float2 cxy = __fmul2_rn(__fadd2_rn(px.xy, make_float2(-s.dist_lo[0], -s.dist_lo[1])), f2(s.dist_inv_cell));
+    const uint32_t ix = (uint32_t)__float2int_rd(cxy.x), iy = (uint32_t)__float2int_rd(cxy.y),
+                   iz = (uint32_t)__float2int_rd(__fmul_rn(__fsub_rn(px.z, s.dist_lo[2]), s.dist_inv_cell));
+    const V3 x = v3(px);
     GridFetch g;
     g.raw = 0xffffu;  // (x q: beyond every stored value -- the box does not bound this point, `other` does)
     g.other = __int_as_float(0x7f800000);
@@ -155,11 +158,11 @@ BT_DEV float grid_bound_finish(const RenderParams& p, const GridFetch& g, float 
 // along a large surface (the r = 100 ground sphere, a unit or three below most of every path) keeps its
 // free distance instead of spending it after a few steps (C3: 23.7 -> 12.8 intersection passes per path, cloud + lens 28.6 -> 18.8).
 template <bool EXACT, int C, class L>
-BT_DEV int geodesic_step(const RenderParams& p, const L& lens, const float4* prims, V3& x, V3& v, Flight& f, float tmax) {
+BT_DEV int geodesic_step(const RenderParams& p, const L& lens, const float4* prims, P3& x, P3& v, Flight& f, float tmax) {
     float rmin;
     bool captured, far;
     D0Cache<L> cache;
-    const V3 k1 = lens_accel<2, EXACT, 0>(lens, cache, x, 0.0f, v, v, rmin, captured, far);
+    const P3 k1 = lens_accel<2, EXACT, 0>(lens, cache, x, 0.0f, v, v, rmin, captured, far);
     if (captured) return FL_CAPTURED;
     if (far) return FL_PEND_FAR;
     // the chord's start is kept where a pending chord needs it (f.xp): the step writes the new position into x and nothing
@@ -178,7 +181,7 @@ BT_DEV int geodesic_step(const RenderParams& p, const L& lens, const float4* pri
     } else if ((C & CT_SPHERES) && f.near >= 0) {
         const float4* q = prims + f.near * PRIM_STRIDE;
         const float4 q0 = q[0], q1 = q[1];
-        const V3 oc = f.xp - v3(q0);
+        const V3 oc = v3(f.xp) - v3(q0);
         free = fminf(sphere_free_bound(q0, q1, fmaf(oc.z, oc.z, fmaf(oc.y, oc.y, oc.x * oc.x))), f.rest);
     }
     rk4_from_k1<EXACT>(lens, cache, x, v, k1, step_size(p.scene.kappa, p.scene.h_min, p.scene.h_max, rmin));
@@ -197,11 +200,11 @@ BT_DEV int geodesic_step(const RenderParams& p, const L& lens, const float4* pri
 // INTERSECTION phase: the pending chord (or the final straight segment) against the scene; the
 // same pass refreshes the free distance.  Returns a resolved state or FL_FLY.
 template <bool EXACT, bool BVH, int C = CT_ALL>
-BT_DEV int geodesic_scan(const RenderParams& p, const SceneView& sc, V3 x, V3 v, Flight& f, int state, float tmin, float tmax) {
+BT_DEV int geodesic_scan(const RenderParams& p, const SceneView& sc, P3 x, P3 v, Flight& f, int state, float tmin, float tmax) {
     const bool far = state == FL_PEND_FAR;
     const float remaining = tmax - f.travelled;
     const float cmin = fmaxf(tmin - f.travelled, 0.0f);
-    const V3 o = far ? x : f.xp;
+    const V3 o = v3(far ? x : f.xp);
     float len;
     const V3 dir = normalize_fma<EXACT>(far ? v : x - f.xp, &len);
     const float cmax = far ? remaining : fminf(len, remaining);
@@ -226,10 +229,10 @@ BT_DEV int geodesic_scan(const RenderParams& p, const SceneView& sc, V3 x, V3 v,
 }
 // the event of a resolved flight
 template <bool EXACT>
-BT_DEV Traced flight_result(int state, V3 x, V3 v, const Flight& f) {
+BT_DEV Traced flight_result(int state, P3 x, P3 v, const Flight& f) {
     Traced r;
     const bool chord = state == FL_HIT;
-    r.o = chord ? f.xp : x;
+    r.o = v3(chord ? f.xp : x);
     r.d = normalize_fma<EXACT>(chord ? x - f.xp : v, 0);
     r.h = f.h;
     if (state >= FL_ESCAPED) r.h.prim = -1;
@@ -247,13 +250,14 @@ BT_DEV Traced trace_ray(const RenderParams& p, const SceneView& sc, const L& len
     if (!LENS || vol_obj >= 0) return trace_straight<BVH>(p, sc, o, d, tmin, tmax, vol_obj);
     Flight f;
     flight_reset(f);
+    P3 x = p3(o), v = p3(d);
     int st = FL_FLY;
 #pragma unroll 1
     while (st < FL_HIT) {
-        st = geodesic_step<EXACT, CT_ALL>(p, lens, sc.prims, o, d, f, tmax);
-        if (st == FL_PEND || st == FL_PEND_FAR) st = geodesic_scan<EXACT, BVH>(p, sc, o, d, f, st, tmin, tmax);
+        st = geodesic_step<EXACT, CT_ALL>(p, lens, sc.prims, x, v, f, tmax);
+        if (st == FL_PEND || st == FL_PEND_FAR) st = geodesic_scan<EXACT, BVH>(p, sc, x, v, f, st, tmin, tmax);
     }
-    return flight_result<EXACT>(st, o, d, f);
+    return flight_result<EXACT>(st, x, v, f);
 }
 
 // NL: 0 = lens table walked in shared memory, N > 0 = exactly N masses held in registers
@@ -648,17 +652,18 @@ BT_DEV void render_body(const RenderParams& p) {
             int ls = !alive ? FL_IDLE : (in_volume ? FL_STRAIGHT : fstate);
             const uint32_t patience = __any_sync(0xffffffffu, ls == FL_STRAIGHT) ? 4u : p.compact_patience;  // straight (volume-march) lanes wait less
             uint32_t waited = 0, scan_waited = 0;
+            P3 x = p3(o), v = p3(d);
 #pragma unroll 1
             for (;;) {
 #pragma unroll 1
                 for (uint32_t r = 0; r < p.steps_per_turn; ++r)  // several steps per turn amortise the ballots below
-                    if (ls == FL_FLY) ls = geodesic_step<EXACT, C>(p, lens, sc.prims, o, d, fl, p.clip_max);
+                    if (ls == FL_FLY) ls = geodesic_step<EXACT, C>(p, lens, sc.prims, x, v, fl, p.clip_max);
                 const bool pend = ls == FL_PEND || ls == FL_PEND_FAR;
                 unsigned m_pend = __ballot_sync(0xffffffffu, pend);
                 unsigned m_fly = __ballot_sync(0xffffffffu, ls == FL_FLY);
                 if (m_pend != 0 && (m_fly == 0 || (uint32_t)__popc(m_pend) >= p.scan_lanes || ++scan_waited >= p.scan_patience)) {
                     scan_waited = 0;
-                    if (pend) ls = geodesic_scan<EXACT, BVH, C>(p, sc, o, d, fl, ls, p.clip_min, p.clip_max);
+                    if (pend) ls = geodesic_scan<EXACT, BVH, C>(p, sc, x, v, fl, ls, p.clip_min, p.clip_max);
                     m_pend = 0;
                     m_fly = __ballot_sync(0xffffffffu, ls == FL_FLY);
                 }
@@ -666,10 +671,12 @@ BT_DEV void render_body(const RenderParams& p) {
                 const unsigned waiting = __ballot_sync(0xffffffffu, (ls & 4) != 0);
                 if (waiting != 0 && ((uint32_t)__popc(waiting) >= p.compact_lanes || ++waited >= patience)) break;
             }
+            o = v3(x);
+            d = v3(v);
             if (ls < FL_IDLE) {
                 fstate = ls;
                 if (ls >= FL_HIT) {
-                    tr = flight_result<EXACT>(ls, o, d, fl);
+                    tr = flight_result<EXACT>(ls, x, v, fl);
                     has_event = true;
                 }
             }
@@ -811,17 +818,17 @@ __global__ void __launch_bounds__(256) integrate_kernel(const __grid_constant__ 
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= p.n) return;
     float* s = p.xv + 6 * (size_t)i;
-    V3 x = v3(s[0], s[1], s[2]), v = v3(s[3], s[4], s[5]);
+    P3 x = p3(make_float2(s[0], s[1]), s[2]), v = p3(make_float2(s[3], s[4]), s[5]);
     const typename LensSel<NL>::type lens = LensSel<NL>::make(slens, (int)p.n_lens);
 #pragma unroll 1
     for (uint32_t it = 0; it < p.n_steps; ++it) {
         float rmin;
         bool captured, far;
         D0Cache<typename LensSel<NL>::type> cache;
-        V3 k1 = lens_accel<1, EXACT, 0>(lens, cache, x, 0.0f, v, v, rmin, captured, far);
+        P3 k1 = lens_accel<1, EXACT, 0>(lens, cache, x, 0.0f, v, v, rmin, captured, far);
         rk4_from_k1<EXACT>(lens, cache, x, v, k1, step_size(p.kappa, p.h_min, p.h_max, rmin));
     }
-    s[0] = x.x; s[1] = x.y; s[2] = x.z; s[3] = v.x; s[4] = v.y; s[5] = v.z;
+    s[0] = x.xy.x; s[1] = x.xy.y; s[2] = x.z; s[3] = v.xy.x; s[4] = v.xy.y; s[5] = v.z;
 }
 
 // Buffer::preview, buffer.rs:117-138

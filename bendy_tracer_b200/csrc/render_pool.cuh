@@ -194,7 +194,7 @@ BT_DEV void render_pool_body(const RenderParams& p) {
             // is paid every other step, not every step.  The phase ends when the stack is empty and fewer
             // lanes fly than another phase has slots waiting.
             int slot = -1, fs = FL_FLY;
-            V3 x = v3(0.0f, 0.0f, 0.0f), v = x;
+            P3 x = p3(make_float2(0.0f, 0.0f), 0.0f), v = x;  // the stepper's paired layout: no conversion per step
             Flight f;
             flight_reset(f);
             uint32_t round_at = 0;  // a refill round runs once this many lanes wait (0: at once)
@@ -209,10 +209,10 @@ BT_DEV void render_pool_body(const RenderParams& p) {
                     const bool left = slot >= 0 && waiting;
                     const bool pend = fs == FL_PEND || fs == FL_PEND_FAR;
                     if (left) {
-                        pl.fa[slot] = make_float4(x.x, x.y, x.z, f.travelled);
-                        pl.fb[slot] = make_float4(v.x, v.y, v.z, f.free);
+                        pl.fa[slot] = make_float4(x.xy.x, x.xy.y, x.z, f.travelled);
+                        pl.fb[slot] = make_float4(v.xy.x, v.xy.y, v.z, f.free);
                         pl.fc[slot] = make_float4(f.rest, __int_as_float(f.near), __uint_as_float(f.steps), 0.0f);
-                        pl.fd[slot] = make_float4(f.xp.x, f.xp.y, f.xp.z, 0.0f);
+                        pl.fd[slot] = make_float4(f.xp.xy.x, f.xp.xy.y, f.xp.z, 0.0f);
                         pl.st[slot] = (uint8_t)(fs + 2);
                     }
                     const uint32_t n_left = __popc(__ballot_sync(0xffffffffu, left)), n_lp = __popc(__ballot_sync(0xffffffffu, left && pend));
@@ -224,8 +224,8 @@ BT_DEV void render_pool_body(const RenderParams& p) {
                     if (waiting && (uint32_t)__popc(m_wait & lt) < take) {
                         slot = pl.stack[n_fly - 1 - __popc(m_wait & lt)];
                         const float4 a = pl.fa[slot], b = pl.fb[slot], c = pl.fc[slot];
-                        x = v3(a);
-                        v = v3(b);
+                        x = p3(a);
+                        v = p3(b);
                         f.travelled = a.w;
                         f.free = b.w;
                         f.rest = c.x;
@@ -254,8 +254,8 @@ BT_DEV void render_pool_body(const RenderParams& p) {
                 const bool fly = slot >= 0;
                 const unsigned m = __ballot_sync(0xffffffffu, fly);
                 if (fly) {
-                    pl.fa[slot] = make_float4(x.x, x.y, x.z, f.travelled);
-                    pl.fb[slot] = make_float4(v.x, v.y, v.z, f.free);
+                    pl.fa[slot] = make_float4(x.xy.x, x.xy.y, x.z, f.travelled);
+                    pl.fb[slot] = make_float4(v.xy.x, v.xy.y, v.z, f.free);
                     pl.fc[slot] = make_float4(f.rest, __int_as_float(f.near), __uint_as_float(f.steps), 0.0f);
                     pl.stack[n_fly + __popc(m & lt)] = (uint8_t)slot;
                 }
@@ -383,8 +383,8 @@ BT_DEV void render_pool_body(const RenderParams& p) {
                     f.near = -1;
                     f.steps = __float_as_uint(c.z);
                     f.scans = 0;
-                    f.xp = v3(e);
-                    const int fs = geodesic_scan<EXACT, false, C>(p, sc, x, v, f, s - 2, p.clip_min, p.clip_max);
+                    f.xp = p3(e);
+                    const int fs = geodesic_scan<EXACT, false, C>(p, sc, p3(x), p3(v), f, s - 2, p.clip_min, p.clip_max);
                     pl.fa[slot].w = f.travelled;
                     if (fs == FL_FLY) {
                         pl.fb[slot].w = f.free;
@@ -440,8 +440,8 @@ BT_DEV void render_pool_body(const RenderParams& p) {
                     f.scans = 0;
                     f.h.t = c.w;
                     unpack_hit(__float_as_uint(e.w), f.h);
-                    f.xp = v3(e);
-                    tr = flight_result<EXACT>(s - 2, o, d, f);
+                    f.xp = p3(e);
+                    tr = flight_result<EXACT>(s - 2, p3(o), p3(d), f);
                 }
                 PathQ q;
                 {
