@@ -419,13 +419,10 @@ BT_DEV bool box_test(const float4* b, V3 o, V3 d, float tmin, float tmax, float&
 // nearest primitive surface (spheres: ||o - c| - r|; rects: L-infinity distance to the world
 // AABB), minus a margin that covers the rounding of the hit tests themselves -- a ray that starts
 // at `o` cannot be reported as hitting anything within that distance (the stepper's chord skip).
-// C: what the scene contains -- a kernel compiled for a scene without rects carries no rect / box
+// C: what the scene contains (CT_* bits, layout.h) -- a kernel compiled for a scene without rects carries no rect / box
 // code, one without volumetric spheres no march code, one without Glass no Fresnel / refraction.
 // The render loop's body has to stay near the 32 KB instruction cache; every shipped scene gets a
-// variant without the code it cannot reach (kernels.cu: launch_render).
-// CT_AOV: the call renders Output::Albedo / Normal / Depth (the first-hit latches of mod.rs:306-315).
-// CT_CUBOID_LIGHT: a Cuboid carries ObjectFlags::LIGHT (WeightedIndex face pick, cuboid.rs:48-81; generic kernels only).
-enum { CT_SPHERES = 1, CT_RECTS = 2, CT_VOLUMES = 4, CT_METAL = 8, CT_GLASS = 16, CT_AOV = 32, CT_CUBOID_LIGHT = 64, CT_ALL = 127 };
+// variant without the code it cannot reach (variants.h).
 // What a DIST scan learns about the surroundings of the ray's origin: the smallest per-primitive
 // bound, the primitive it belongs to when that is a sphere (-1 otherwise) and the smallest bound among
 // all the other primitives.  The stepper re-evaluates the nearest sphere's distance exactly at every

@@ -8,14 +8,18 @@
 // Pixel sums are formed in the reference's order, so the result is deterministic.
 #include "device.cuh"
 #include "kernels.h"
+#include "variants.h"
 
 #include <algorithm>
 #include <cstdlib>
+#include <utility>
 
 #ifdef BT_EXACT_SCAN
 #define BT_SFX(name) name##_exact
+constexpr bool kExactFlavour = true;
 #else
 #define BT_SFX(name) name##_fast
+constexpr bool kExactFlavour = false;
 #endif
 
 namespace bt {
@@ -720,7 +724,7 @@ BT_DEV void render_body(const RenderParams& p) {
 
 // Lensed variants carry the flight state on top of the path state: 128-thread CTAs at 5 per SM give
 // them 96 registers (20 warps / SM) instead of 80 with spills (24 warps / SM).  The flat variants keep
-// the 85-register cap of (256, 3) and are launched with 128 threads as well (launch_render).
+// the 85-register cap of (256, 3) and are launched with 128 threads as well (launch_lane).
 #ifndef BT_BVH_CTAS
 #define BT_BVH_CTAS 7  // (measured 4 .. 7: the traversal is latency-bound, every CTA more is +6 .. +15 %)
 #endif
@@ -915,35 +919,13 @@ size_t render_smem_bytes(const RenderParams& p, unsigned threads) {
 
 #endif
 
-// picks <LENS, EXACT, NL, BVH> from the scene header (TAIL: name of a function-like macro giving further template arguments)
-#define BT_LAUNCH_(KERNEL, L, E, N, B, TAIL, GRID, BLOCK, SMEM, STREAM, ...)                           \
-    do {                                                                                              \
-        cudaError_t e_ = ensure_smem(KERNEL<L, E, N, B TAIL()>, SMEM);                                   \
-        if (e_ != cudaSuccess) return e_;                                                              \
-        KERNEL<L, E, N, B TAIL()><<<GRID, BLOCK, SMEM, STREAM>>>(__VA_ARGS__);                           \
-    } while (0)
-#define BT_TAIL_NONE()
-#define BT_TAIL_NO_CUBOID_LIGHT() , (CT_ALL & ~CT_CUBOID_LIGHT)
-#define BT_DISPATCH_LENS(KERNEL, TAIL, GRID, BLOCK, SMEM, STREAM, ...)                                 \
-    do {                                                                                              \
-        const bool exact_ = p.scene.lens_exact != 0, bvh_ = p.scene.n_bvh != 0;                        \
-        if (p.scene.n_lens == 0 && !bvh_) BT_LAUNCH_(KERNEL, false, false, 0, false, TAIL, GRID, BLOCK, SMEM, STREAM, __VA_ARGS__);      \
-        else if (p.scene.n_lens == 0) BT_LAUNCH_(KERNEL, false, false, 0, true, TAIL, GRID, BLOCK, SMEM, STREAM, __VA_ARGS__);           \
-        else if (bvh_ && exact_) BT_LAUNCH_(KERNEL, true, true, 0, true, TAIL, GRID, BLOCK, SMEM, STREAM, __VA_ARGS__);                   \
-        else if (bvh_) BT_LAUNCH_(KERNEL, true, false, 0, true, TAIL, GRID, BLOCK, SMEM, STREAM, __VA_ARGS__);                            \
-        else if (p.scene.n_lens == 1 && !exact_) BT_LAUNCH_(KERNEL, true, false, 1, false, TAIL, GRID, BLOCK, SMEM, STREAM, __VA_ARGS__); \
-        else if (!exact_) BT_LAUNCH_(KERNEL, true, false, 0, false, TAIL, GRID, BLOCK, SMEM, STREAM, __VA_ARGS__);                        \
-        else BT_LAUNCH_(KERNEL, true, true, 0, false, TAIL, GRID, BLOCK, SMEM, STREAM, __VA_ARGS__);                                      \
-    } while (0)
-
 namespace {
-// persistent grid of the pooled kernel: as many CTAs as fit the GPU at once (each warp walks the tiles
-// g, g + G, ...), or fewer when the frame has fewer 8 x 4 tiles than that
+// persistent grid of the pooled kernel: as many CTAs as fit the GPU at once, or fewer when the frame has fewer
+// 8 x 4 tiles than that (the warps draw their tiles from one counter: render_pool.cuh)
 template <class K>
-cudaError_t launch_pool(K kernel, const RenderParams& p, bool lens, bool aov, cudaStream_t stream) {
+cudaError_t launch_pool(K kernel, const RenderParams& p, bool lens, cudaStream_t stream) {
     const unsigned cap = 128;  // BT_POOL_BOUNDS
     const unsigned threads = p.pool_threads ? std::min(p.pool_threads, cap) : cap, warps = threads / 32;
-    (void)aov;
     const bool bvh = p.scene.n_bvh != 0;
     const size_t smem = (size_t)p.scene.stage_f4 * sizeof(float4) + warps * pool_warp_bytes(p.pool_w, lens, bvh);
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -961,119 +943,64 @@ cudaError_t launch_pool(K kernel, const RenderParams& p, bool lens, bool aov, cu
     kernel<<<(unsigned)std::max<uint64_t>(1, std::min(std::min(need, fit), room)), threads, smem, stream>>>(p);
     return cudaGetLastError();
 }
+
+// the lane kernels: a CTA renders 16 x (threads / 16) pixels.  128-thread CTAs (16 x 8 pixels): at <= 72 registers seven
+// of them fit an SM (28 warps) where three 256-thread CTAs gave 24 -- cornell2 +3.7 % (the work-counter variant keeps 256)
+template <class K>
+cudaError_t launch_lane(K kernel, const RenderParams& p, unsigned threads, cudaStream_t stream) {
+    const uint32_t rows = p.row_end - p.row0, h = threads / 16;
+    const size_t smem = render_smem_bytes(p, threads);
+    cudaError_t e = ensure_smem(kernel, smem);
+    if (e != cudaSuccess) return e;
+    kernel<<<dim3((p.width + 15) / 16, (rows + h - 1) / h), threads, smem, stream>>>(p);
+    return cudaGetLastError();
+}
+
+struct TraceArgs { uint32_t n; const float *origins, *dirs; DeviceSegment* out; };
+
+// row I of the variant table (variants.h): the kernels of the families it lists, and nothing else, are instantiated
+template <size_t I>
+cudaError_t launch_variant(int family, const RenderParams& p, const TraceArgs& t, cudaStream_t stream) {
+    constexpr Variant v = kVariants[I];
+    constexpr int F = variant_families(v, kExactFlavour);
+    if constexpr ((F & V_LANE) != 0) if (family == V_LANE) return launch_lane(render_kernel<v.lens, v.exact, v.nl, v.bvh, v.c>, p, 128, stream);
+    if constexpr ((F & V_LANE_STATS) != 0) if (family == V_LANE_STATS) return launch_lane(render_kernel_stats<v.lens, v.exact, v.nl, v.bvh, v.c>, p, 256, stream);
+    if constexpr ((F & V_POOL) != 0) if (family == V_POOL) return launch_pool(render_pool_kernel<v.lens, v.exact, v.nl, v.c>, p, v.lens, stream);
+    if constexpr ((F & V_POOL_STATS) != 0) if (family == V_POOL_STATS) return launch_pool(render_pool_kernel_pstats<v.lens, v.exact, v.nl, v.c>, p, v.lens, stream);
+    if constexpr ((F & V_POOL_BVH) != 0) if (family == V_POOL_BVH) return launch_pool(render_pool_bvh_kernel<v.c>, p, false, stream);
+    if constexpr ((F & V_TRACE) != 0) if (family == V_TRACE) {
+        const size_t smem = render_smem_bytes(p);
+        cudaError_t e = ensure_smem(trace_kernel<v.lens, v.exact, v.nl, v.bvh>, smem);
+        if (e != cudaSuccess) return e;
+        trace_kernel<v.lens, v.exact, v.nl, v.bvh><<<(t.n + 255) / 256, 256, smem, stream>>>(p, t.n, t.origins, t.dirs, t.out);
+        return cudaGetLastError();
+    }
+    return cudaErrorNotSupported;
+}
+
+template <size_t... I>
+cudaError_t launch_row(int row, int family, const RenderParams& p, const TraceArgs& t, cudaStream_t stream, std::index_sequence<I...>) {
+    static constexpr cudaError_t (*rows[])(int, const RenderParams&, const TraceArgs&, cudaStream_t) = {&launch_variant<I>...};
+    return rows[row](family, p, t, stream);
+}
+
+// a call no row serves is an error (bt_render_pool_stats: BT_ERR_UNSUPPORTED), never a fall-back to another family
+cudaError_t launch_family(int family, const RenderParams& p, const TraceArgs& t, cudaStream_t stream, uint64_t* launches) {
+    const int row = select_variant(p, family, kExactFlavour);
+    if (row < 0) return cudaErrorNotSupported;
+    ++*launches;
+    return launch_row(row, family, p, t, stream, std::make_index_sequence<kNumVariants>());
+}
 }  // namespace
 
 cudaError_t BT_SFX(launch_render)(const RenderParams& p, cudaStream_t stream, uint64_t* launches) {
-    // (the pooled kernel packs a path's counters into 8 bits each and its volume object into 7: render_pool.cuh)
-    const bool bvh_pool = p.scene.n_bvh != 0 && p.scene.n_lens == 0;  // (no volumetric spheres under a BVH: nothing to pack)
-    const bool pool_ok = p.pool_w != 0 && (p.scene.n_bvh == 0 || bvh_pool) && p.max_bounces <= POOL_MAX_BOUNCES &&
-                         p.max_volume_bounces <= POOL_MAX_BOUNCES && (p.scene.n_prims <= POOL_MAX_OBJECTS || bvh_pool);
-    if (pool_ok && bvh_pool && !p.stats && !p.pool_stats) {
-        const uint32_t ct = p.scene.content | (p.output != 0 ? (uint32_t)CT_AOV : 0u);
-        cudaError_t e_;
-        if (ct & CT_CUBOID_LIGHT) e_ = launch_pool(render_pool_bvh_kernel<CT_ALL>, p, false, true, stream);
-        else e_ = launch_pool(render_pool_bvh_kernel<CT_ALL & ~CT_CUBOID_LIGHT>, p, false, true, stream);
-        ++*launches;
-        return e_;
-    }
-    if (pool_ok && !bvh_pool && p.pool_stats) {
-        const uint32_t ct = p.scene.content;
-        const bool lensed = p.scene.n_lens != 0, ok = p.output == 0 && !(lensed && (p.scene.lens_exact || p.scene.n_lens != 1));
-#define BT_FITS_(C) ((ct & ~(uint32_t)(C)) == 0)
-#define BT_POOL_(L, E, N, C) e_ = launch_pool(render_pool_kernel_pstats<L, E, N, C>, p, L, false, stream)
-        cudaError_t e_ = cudaErrorNotSupported;
-        if (ok && !lensed && BT_FITS_(CT_RECTS)) BT_POOL_(false, false, 0, CT_RECTS);
-        else if (ok && !lensed && BT_FITS_(CT_RECTS | CT_METAL)) BT_POOL_(false, false, 0, CT_RECTS | CT_METAL);
-        else if (ok && !lensed && BT_FITS_(CT_SPHERES | CT_VOLUMES)) BT_POOL_(false, false, 0, CT_SPHERES | CT_VOLUMES);
-        else if (ok && !lensed && BT_FITS_(CT_SPHERES | CT_METAL | CT_GLASS)) BT_POOL_(false, false, 0, CT_SPHERES | CT_METAL | CT_GLASS);
-        else if (ok && lensed && BT_FITS_(CT_SPHERES | CT_METAL | CT_GLASS)) BT_POOL_(true, false, 1, CT_SPHERES | CT_METAL | CT_GLASS);
-        else if (ok && lensed && BT_FITS_(CT_SPHERES | CT_VOLUMES)) BT_POOL_(true, false, 1, CT_SPHERES | CT_VOLUMES);
-        else if (p.output == 0 && lensed && p.scene.n_lens == 1 && p.scene.lens_exact && BT_FITS_(CT_SPHERES | CT_VOLUMES))
-            BT_POOL_(true, true, 1, CT_SPHERES | CT_VOLUMES);
-#undef BT_POOL_
-#undef BT_FITS_
-        ++*launches;
-        return e_;
-    }
-    if (pool_ok && !bvh_pool && !p.stats) {
-        // the pooled kernel (render_pool.cuh): the same variants as below
-        const uint32_t ct = p.scene.content | (p.output != 0 ? (uint32_t)CT_AOV : 0u);
-        const bool lensed = p.scene.n_lens != 0, one = p.scene.n_lens == 1, exact = p.scene.lens_exact != 0;
-        const bool special = !(lensed && (exact || !one));
-#define BT_FITS_(C) ((ct & ~(uint32_t)(C)) == 0)
-#define BT_POOL_(L, E, N, C) e_ = launch_pool(render_pool_kernel<L, E, N, C>, p, L, ((C) & CT_AOV) != 0, stream)
-        cudaError_t e_;
-        if (special && !lensed && BT_FITS_(CT_RECTS)) BT_POOL_(false, false, 0, CT_RECTS);
-        else if (special && !lensed && BT_FITS_(CT_RECTS | CT_METAL)) BT_POOL_(false, false, 0, CT_RECTS | CT_METAL);
-        else if (special && !lensed && BT_FITS_(CT_SPHERES | CT_VOLUMES)) BT_POOL_(false, false, 0, CT_SPHERES | CT_VOLUMES);
-        else if (special && !lensed && BT_FITS_(CT_SPHERES | CT_METAL | CT_GLASS)) BT_POOL_(false, false, 0, CT_SPHERES | CT_METAL | CT_GLASS);
-        else if (special && lensed && BT_FITS_(CT_SPHERES | CT_METAL | CT_GLASS)) BT_POOL_(true, false, 1, CT_SPHERES | CT_METAL | CT_GLASS);
-        else if (special && lensed && BT_FITS_(CT_SPHERES | CT_VOLUMES)) BT_POOL_(true, false, 1, CT_SPHERES | CT_VOLUMES);
-        else if (lensed && one && exact && BT_FITS_(CT_SPHERES | CT_VOLUMES)) BT_POOL_(true, true, 1, CT_SPHERES | CT_VOLUMES);  // cloud / volume + one mass, exact stepper
-        else if (ct & CT_CUBOID_LIGHT) {
-            if (!lensed) BT_POOL_(false, false, 0, CT_ALL);
-            else if (exact) BT_POOL_(true, true, 0, CT_ALL);
-            else if (one) BT_POOL_(true, false, 1, CT_ALL);
-            else BT_POOL_(true, false, 0, CT_ALL);
-        } else {
-            if (!lensed) BT_POOL_(false, false, 0, CT_ALL & ~CT_CUBOID_LIGHT);
-            else if (exact) BT_POOL_(true, true, 0, CT_ALL & ~CT_CUBOID_LIGHT);
-            else if (one) BT_POOL_(true, false, 1, CT_ALL & ~CT_CUBOID_LIGHT);
-            else BT_POOL_(true, false, 0, CT_ALL & ~CT_CUBOID_LIGHT);
-        }
-#undef BT_POOL_
-#undef BT_FITS_
-        ++*launches;
-        return e_;
-    }
-    // 128-thread CTAs (16 x 8 pixels): at <= 72 registers seven of them fit an SM (28 warps) where three
-    // 256-thread CTAs gave 24 -- cornell2 +3.7 % (the work-counter variant keeps 256 threads)
-    const bool small = !p.stats;
-    const uint32_t rows = p.row_end - p.row0;
-    dim3 grid((p.width + 15) / 16, small ? (rows + 7) / 8 : (rows + 15) / 16), block(small ? 128 : 256);
-    size_t smem = render_smem_bytes(p, block.x);
-    // content-specialised variants (device.cuh CT_*): the smallest compiled superset of what the scene holds
-#define BT_LAUNCH_C_(L, N, C)                                                                          \
-    do {                                                                                               \
-        cudaError_t e_ = ensure_smem(render_kernel<L, false, N, false, C>, smem);                      \
-        if (e_ != cudaSuccess) return e_;                                                              \
-        render_kernel<L, false, N, false, C><<<grid, block, smem, stream>>>(p);                        \
-    } while (0)
-    const uint32_t ct = p.scene.content | (p.output != 0 ? (uint32_t)CT_AOV : 0u);
-    const bool plain = !p.stats && p.scene.n_bvh == 0 && !(p.scene.n_lens != 0 && (p.scene.lens_exact || p.scene.n_lens != 1));
-    const bool lensed = p.scene.n_lens != 0;
-#define BT_FITS_(C) ((ct & ~(uint32_t)(C)) == 0)
-    if (plain && !lensed && BT_FITS_(CT_RECTS))
-        BT_LAUNCH_C_(false, 0, CT_RECTS);                                    // cornell.json.gz
-    else if (plain && !lensed && BT_FITS_(CT_RECTS | CT_METAL))
-        BT_LAUNCH_C_(false, 0, CT_RECTS | CT_METAL);                         // cornell2.json.gz
-    else if (plain && !lensed && BT_FITS_(CT_SPHERES | CT_VOLUMES))
-        BT_LAUNCH_C_(false, 0, CT_SPHERES | CT_VOLUMES);                     // cloud / volume.json.gz
-    else if (plain && !lensed && BT_FITS_(CT_SPHERES | CT_METAL | CT_GLASS))
-        BT_LAUNCH_C_(false, 0, CT_SPHERES | CT_METAL | CT_GLASS);            // scene.json.gz
-    else if (plain && lensed && BT_FITS_(CT_SPHERES | CT_METAL | CT_GLASS))
-        BT_LAUNCH_C_(true, 1, CT_SPHERES | CT_METAL | CT_GLASS);             // scene.json.gz + one mass (C3 / C5)
-    else if (plain && lensed && BT_FITS_(CT_SPHERES | CT_VOLUMES))
-        BT_LAUNCH_C_(true, 1, CT_SPHERES | CT_VOLUMES);                      // cloud / volume + one mass
-    else if (p.stats)
-        BT_DISPATCH_LENS(render_kernel_stats, BT_TAIL_NONE, grid, block, smem, stream, p);
-    else if (ct & CT_CUBOID_LIGHT)  // a LIGHT Cuboid: the only content that needs the WeightedIndex / Cuboid::pdf code
-        BT_DISPATCH_LENS(render_kernel, BT_TAIL_NONE, grid, block, smem, stream, p);
-    else
-        BT_DISPATCH_LENS(render_kernel, BT_TAIL_NO_CUBOID_LIGHT, grid, block, smem, stream, p);
-#undef BT_FITS_
-#undef BT_LAUNCH_C_
-    ++*launches;
-    return cudaGetLastError();
+    return launch_family(render_family(p), p, TraceArgs{}, stream, launches);
 }
 
 cudaError_t BT_SFX(launch_trace)(const RenderParams& p, uint32_t n, const float* origins, const float* dirs,
                          DeviceSegment* out, cudaStream_t stream, uint64_t* launches) {
     if (n == 0) return cudaSuccess;
-    size_t smem = render_smem_bytes(p);
-    BT_DISPATCH_LENS(trace_kernel, BT_TAIL_NONE, (n + 255) / 256, 256, smem, stream, p, n, origins, dirs, out);
-    ++*launches;
-    return cudaGetLastError();
+    return launch_family(V_TRACE, p, TraceArgs{n, origins, dirs, out}, stream, launches);
 }
 
 cudaError_t BT_SFX(launch_camera_rays)(const RenderParams& p, uint32_t n, const uint32_t* xs, const uint32_t* ys,

@@ -74,6 +74,11 @@ enum { BOX_STRIDE = 4 };
 //   b0 = (lo.xyz, -)   b1 = (hi.xyz, -)   world AABB of a rect; unused for spheres (exact formula)
 enum { BOUND_STRIDE = 2 };
 
+// ---- content bits: SceneHeader::content, and the template mask C of the kernel variants (variants.h)
+// CT_AOV: the call renders Output::Albedo / Normal / Depth (the first-hit latches of mod.rs:306-315).
+// CT_CUBOID_LIGHT: a Cuboid carries ObjectFlags::LIGHT (WeightedIndex face pick, cuboid.rs:48-81; generic kernels only).
+enum { CT_SPHERES = 1, CT_RECTS = 2, CT_VOLUMES = 4, CT_METAL = 8, CT_GLASS = 16, CT_AOV = 32, CT_CUBOID_LIGHT = 64, CT_ALL = 127 };
+
 struct SceneHeader {
     uint32_t n_prims, prim_off;      // offsets in float4 units into the blob
     uint32_t n_mats, mat_off;
@@ -86,7 +91,7 @@ struct SceneHeader {
     uint32_t n_bvh, bvh_off;         // BVH nodes (0: linear scan over shared memory)
     uint32_t stage_off, stage_f4;    // the part of the blob every CTA stages into shared memory
     uint32_t has_volume_prims;       // any sphere with volume != None
-    uint32_t content;                // CT_* bits (device.cuh): picks a kernel without the unused code
+    uint32_t content;                // CT_* bits of the scene (CT_AOV comes from the call): picks a kernel without the unused code
     // root material folded to what sample_root returns (src/tracer/mod.rs:429-452)
     float root_color[3], root_albedo[3];
     uint32_t root_keeps_normal;      // 1: normal = -dir, depth = clip_max; 0: normal = 0, depth = inf

@@ -57,9 +57,8 @@ struct Pool {
     uint8_t *st, *list, *stack, *ring;
     unsigned long long* tiles;  // the warp's window of tile indices: tile k of its stream is tiles[k % POOL_TILES]
 };
-// misc packs the counters of a path into 8 bits each: the pooled kernel serves max_bounces, max_volume_bounces <= POOL_MAX_BOUNCES
-// and scenes of up to 126 objects (launch_render falls back to render_body otherwise)
-enum { POOL_MAX_BOUNCES = 254, POOL_MAX_OBJECTS = 126 };
+// misc packs the counters of a path into 8 bits each: the pooled kernel serves the calls within POOL_MAX_BOUNCES and
+// POOL_MAX_OBJECTS (variants.h: render_family; the lane kernel renders the others)
 BT_DEV uint32_t pack_misc(uint32_t ring, bool latched, int vol_obj, uint32_t bounce, uint32_t vb) {
     return ring | (latched ? 16u : 0u) | ((uint32_t)(vol_obj + 1) << 5) | (bounce << 12) | (vb << 20);
 }

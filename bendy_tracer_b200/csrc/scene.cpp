@@ -1408,7 +1408,7 @@ FlatScene flatten(const Scene& scene, int accel) {
                 lights[base + 2].z = as_f((uint32_t)(face_lights.size() / LIGHT_STRIDE));
                 cuboid_lights.push_back(base);
                 face_lights.insert(face_lights.end(), rec.face_lights.begin(), rec.face_lights.end());
-                fs.header.content |= 64u;  // CT_CUBOID_LIGHT
+                fs.header.content |= CT_CUBOID_LIGHT;
                 if (rec.zero_area) fs.cuboid_light_without_area = true;  // WeightedIndex::new(..).unwrap() panics
             }
         }
@@ -1438,17 +1438,17 @@ FlatScene flatten(const Scene& scene, int accel) {
     h.n_vols = (uint32_t)(vols.size() / VOL_STRIDE);
     h.n_lens = (uint32_t)(lens.size() / LENS_STRIDE);
     h.prim_off = 0;
-    h.content &= 64u;  // (CT_CUBOID_LIGHT was set while flattening the lights)
+    h.content &= CT_CUBOID_LIGHT;  // (set while flattening the lights)
     for (uint32_t i = 0; i < h.n_prims; ++i) {
         uint32_t type;
         std::memcpy(&type, &prims[(size_t)i * PRIM_STRIDE + 4].x, 4);
-        h.content |= (type & 3u) == PRIM_SPHERE ? 1u : 2u;
+        h.content |= (type & 3u) == PRIM_SPHERE ? CT_SPHERES : CT_RECTS;
     }
-    if (h.has_volume_prims) h.content |= 4u;
+    if (h.has_volume_prims) h.content |= CT_VOLUMES;
     for (std::map<uint64_t, Data>::const_iterator it = scene.data.begin(); it != scene.data.end(); ++it) {
         if (it->second.kind != DATA_MATERIAL) continue;
-        if (it->second.mat_kind == MAT_METALLIC) h.content |= 8u;
-        if (it->second.mat_kind == MAT_GLASS) h.content |= 16u;
+        if (it->second.mat_kind == MAT_METALLIC) h.content |= CT_METAL;
+        if (it->second.mat_kind == MAT_GLASS) h.content |= CT_GLASS;
     }
     // acceleration structure: the linear scan of the reference for small scenes, a BVH beyond
     bool use_bvh = accel == ACCEL_BVH || (accel == ACCEL_AUTO && h.n_prims > (uint32_t)BVH_AUTO_PRIMS);

@@ -244,8 +244,9 @@ int bt_render_stats(bt_engine* engine, bt_scene* scene, uint64_t camera_ref, con
  * stats_out = {STEP iterations, flying lanes summed over them, refill rounds, STEP entries, SCAN passes,
  * slots scanned, SHADE passes, slots shaded, REGEN passes, paths issued, paths retired, turns, SM clocks the
  * warps spent in STEP, SCAN, SHADE, REGEN, SM clocks of the warps' whole lives} summed over all warps -- lanes
- * per pass = slots / passes.  BT_ERR_UNSUPPORTED when pool_w = 0 or the scene runs a
- * generic (not content-specialised) kernel. */
+ * per pass = slots / passes.  BT_ERR_UNSUPPORTED when no content-specialised pooled kernel renders the
+ * call: pool_w = 0, a BVH scene, max bounces above 254, more than 126 primitives, or a scene or output
+ * that only a generic kernel serves. */
 int bt_render_pool_stats(bt_engine* engine, bt_scene* scene, uint64_t camera_ref, const bt_config* config,
                          const bt_render_config* render_config, uint64_t seed, uint64_t sample_base,
                          uint32_t width, uint32_t height, uint64_t stats_out[17]);

@@ -203,3 +203,27 @@ def test_pool_bvh_traversal_equals_lane_kernel(precision):
                 assert np.array_equal(got, ref), (pool_w, "bvh_stack_k=1")
             else:
                 assert (np.abs(got - ref).mean(axis=(0, 1)) / 8 <= 1e-6).all(), pool_w
+
+
+def test_pool_stats_only_from_the_pooled_kernel():
+    """bt_render_pool_stats reports the pooled kernel's scheduling counters, or BT_ERR_UNSUPPORTED when the call would not run
+    a content-specialised pooled kernel: a BVH scene, or max_bounces beyond the pooled kernel's packed counters"""
+    import json
+
+    import bendy_tracer_b200 as bt
+    from common import synthetic_scene
+    w, h, passes = 64, 32, 2
+    rc = bt.RenderConfig.with_samples_subsample(passes, bt.Subsample(2))
+    sc, cam = _scene("scene", w, h, LENS_SCENE)
+    stats = bt.Tracer(bt.Config(), seed=1).render_pool_stats(sc, cam, rc, w, h)
+    assert stats["paths_issued"] == stats["paths_retired"] == w * h * passes * 4
+    with pytest.raises(bt.BendyError) as e:
+        bt.Tracer(bt.Config(max_bounces=300), seed=1).render_pool_stats(sc, cam, rc, w, h)
+    assert e.value.code == bt._ffi.ERR_UNSUPPORTED
+    bvh = bt.Scene.from_json(json.dumps(synthetic_scene()))
+    assert bvh.info()["n_bvh_nodes"] > 0
+    cam = bvh.find_by_tag("camera")
+    bvh.set_camera_aspect(cam, float(np.float32(w) / np.float32(h)))
+    with pytest.raises(bt.BendyError) as e:
+        bt.Tracer(bt.Config(), seed=1).render_pool_stats(bvh, cam, rc, w, h)
+    assert e.value.code == bt._ffi.ERR_UNSUPPORTED
