@@ -59,6 +59,7 @@ SIGNATURES = {
     "bt_scene_destroy": (None, [_P]),
     "bt_scene_find_by_tag": (C.c_int, [_P, C.c_char_p, C.POINTER(C.c_uint64)]),
     "bt_scene_set_camera_aspect": (C.c_int, [_P, C.c_uint64, C.c_float]),
+    "bt_scene_set_camera_projection": (C.c_int, [_P, C.c_uint64, C.c_int]),
     "bt_scene_apply_transform": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_float)]),
     "bt_scene_commit": (C.c_int, [_P]),
     "bt_scene_set_lenses": (C.c_int, [_P, _P, C.c_uint32, C.POINTER(BtLensConfig)]),

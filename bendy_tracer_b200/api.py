@@ -29,6 +29,13 @@ class Output(enum.IntEnum):
     Depth = 3
 
 
+class Projection(enum.IntEnum):
+    """camera projection (extension, bt_scene_set_camera_projection): the reference's frustum, or the whole sphere around
+    the camera in the environment map's equirectangular convention"""
+    PERSPECTIVE = 0
+    EQUIRECTANGULAR = 1
+
+
 class Status(enum.IntEnum):
     """reference src/tracer/mod.rs:159-163"""
     Done = 0
@@ -250,6 +257,12 @@ class Scene:
     def set_camera_aspect(self, camera_ref, aspect_ratio):
         """the update main pushes through its UpdateQueue (src/main.rs:218-223)"""
         check(lib.bt_scene_set_camera_aspect(self.handle, camera_ref, aspect_ratio))
+
+    def set_camera_projection(self, camera_ref, projection):
+        """Projection.PERSPECTIVE (the default) or Projection.EQUIRECTANGULAR: a pinhole panorama of the whole sphere, pixel
+        (x, y) looking at the centre of texel (x, y) of a map of the image's size (bt_scene_set_camera_projection).  Not part
+        of the wire format.  A non-camera reference raises ScenePanic, an unknown projection BendyError"""
+        check(lib.bt_scene_set_camera_projection(self.handle, camera_ref, int(projection)))
 
     def apply_transform(self, object_ref, affine):
         """Object::apply_transform + UpdateQueue::commit (src/scene/object/mod.rs:212-223)"""

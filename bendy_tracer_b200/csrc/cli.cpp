@@ -3,7 +3,8 @@
 //
 //   bendy_b200_cli --output full|albedo|normal [--width 768] [--height 512] [--samples 64]
 //                  [--subsample 2] [--screenshot screenshots/render.png] [--scene scene.json]
-//                  [--lens x,y,z,r_s] [--environment sky.pfm] [--seed 0] [--save-scene out.json(.gz)]
+//                  [--lens x,y,z,r_s] [--environment sky.pfm] [--projection perspective|equirectangular]
+//                  [--seed 0] [--save-scene out.json(.gz)]
 //
 // Same flags, defaults and semantics as the reference's clap CLI: `--output` is required; the scene
 // file is read when it exists (gzip when the extension is .gz), otherwise the built-in Cornell box
@@ -13,7 +14,9 @@
 // is written as PNG (what Ctrl+P does, main.rs:275-298).  Instead of the title bar the per-pass
 // time, average and total are printed to stderr (main.rs:352-388).  --environment (an extension, like --lens) sets an
 // equirectangular environment map from a PFM file (bt_scene_set_environment); a malformed file is an error even in the
-// GPU-less --samples 0 dry run.
+// GPU-less --samples 0 dry run.  --projection equirectangular (an extension too) renders the whole sphere around the
+// camera (bt_scene_set_camera_projection; --width = 2 --height gives square pixels); an unknown value is an error before
+// any GPU work.
 #include <zlib.h>
 
 #include <cctype>
@@ -200,7 +203,7 @@ std::vector<float> read_pfm(const std::string& path, uint32_t* w_out, uint32_t* 
 int main(int argc, char** argv) {
     uint32_t width = 768, height = 512, subsample = 2;
     uint64_t samples = 64, seed = 0;
-    int output = -1;
+    int output = -1, projection = BT_PROJECTION_PERSPECTIVE;
     std::string screenshot = "screenshots/render.png", scene_path = "scene.json", save_scene, environment;
     std::vector<float> lens;
     for (int i = 1; i < argc; ++i) {
@@ -218,6 +221,11 @@ int main(int argc, char** argv) {
         else if (a == "--scene") scene_path = val();
         else if (a == "--save-scene") save_scene = val();
         else if (a == "--environment") environment = val();
+        else if (a == "--projection") {
+            std::string v = val();
+            projection = v == "perspective" ? BT_PROJECTION_PERSPECTIVE : v == "equirectangular" ? BT_PROJECTION_EQUIRECTANGULAR : -1;
+            if (projection < 0) die("invalid value '" + v + "' for '--projection <PROJECTION>' [possible values: perspective, equirectangular]");
+        }
         else if (a == "--lens") {
             std::stringstream ss(val());
             std::string tok;
@@ -255,6 +263,10 @@ int main(int argc, char** argv) {
     uint64_t camera = 0;
     ck(bt_scene_find_by_tag(scene, "camera", &camera), "find_by_tag(\"camera\")");
     ck(bt_scene_set_camera_aspect(scene, camera, (float)width / (float)height), "camera aspect");  // main.rs:218-223
+    if (projection != BT_PROJECTION_PERSPECTIVE) {
+        ck(bt_scene_set_camera_projection(scene, camera, projection), "camera projection");
+        std::fprintf(stderr, "projection equirectangular: %u x %u\n", width, height);
+    }
     if (!save_scene.empty()) {  // what Ctrl+K does, main.rs:299-313 (plain JSON here)
         char* text = nullptr;
         size_t n = 0;

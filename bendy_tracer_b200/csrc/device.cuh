@@ -204,11 +204,8 @@ BT_DEV uint32_t uniform_index(Rng& rng, uint32_t n, uint64_t zone) {
 // parts and the Cephes single-precision minimax polynomials on [-pi/4, pi/4], all in explicit FMAs.
 // <= 1.5 ulp, like CUDA's sincosf, at a quarter of its code size (no Payne-Hanek path): the render
 // kernel calls it from four places and its loop body has to stay inside the instruction cache.
-BT_DEV void bt_sincos(float x, float* sn, float* cs) {
-#ifdef BT_EXACT_SCAN
-    sincosf(x, sn, cs);  // agrees with glibc's sinf / cosf (the oracle) on all but ~1e-4 of arguments
-    return;
-#endif
+// Every operation is IEEE (explicit FMAs, rintf), so a CPU repeats it bit for bit (tests/oracle_camera.cpp).
+BT_DEV void sincos_poly(float x, float* sn, float* cs) {
     const float k = rintf(x * 0.636619772367581343f);
     float y = fmaf(k, -1.5703125f, x);
     y = fmaf(k, -4.837512969970703125e-4f, y);
@@ -224,6 +221,13 @@ BT_DEV void bt_sincos(float x, float* sn, float* cs) {
     const float a = (q & 1) ? c : s, b = (q & 1) ? s : c;
     *sn = (q & 2) ? -a : a;
     *cs = ((q + 1) & 2) ? -b : b;
+}
+BT_DEV void bt_sincos(float x, float* sn, float* cs) {
+#ifdef BT_EXACT_SCAN
+    sincosf(x, sn, cs);  // agrees with glibc's sinf / cosf (the oracle) on all but ~1e-4 of arguments
+#else
+    sincos_poly(x, sn, cs);
+#endif
 }
 
 struct Consts {  // Uniform::new_inclusive(0, TAU) / (0, 1): low = 0
@@ -907,12 +911,8 @@ BT_DEV V3 env_lookup(const float4* env, uint32_t w, uint32_t h, V3 d) {
 // ------------------------------------------------------------------------------------------
 // camera (mod.rs:272-302, ray.rs:103-137)
 // ------------------------------------------------------------------------------------------
-BT_DEV V3 with_frustum_dir(float yfov, float xfov, float u, float v) {
-    float yrot = xfov * 0.5f * -u;
-    float xrot = yfov * 0.5f * -v;
-    float sy, cy, sx, cx;
-    bt_sincos(yrot * 0.5f, &sy, &cy);
-    bt_sincos(xrot * 0.5f, &sx, &cx);
+// Quat::from_euler(YXZ, yrot, xrot, 0) * NEG_Z from (sin, cos) of yrot / 2 and xrot / 2
+BT_DEV V3 with_frustum_dir(float sy, float cy, float sx, float cx) {
     float qx = cy * sx, qy = sy * cx, qz = -(sy * sx), qw = cy * cx;
     V3 b = v3(qx, qy, qz);
     V3 vv = v3(0.0f, 0.0f, -1.0f);
@@ -922,7 +922,24 @@ BT_DEV V3 with_frustum_dir(float yfov, float xfov, float u, float v) {
     float s3 = qw * 2.0f;
     return (vv * s1 + b * s2) + cross(b, vv) * s3;
 }
-// (sub_i, sub_j): the sub-pixel of this path, i fastest (mod.rs:70-106)
+// camera_ray's sin / cos: the frustum keeps bt_sincos; the panorama takes sincos_poly in both flavours, which the test oracle
+// repeats bit for bit (CUDA's sincosf and glibc's sinf / cosf disagree in some component of ~45 % of panorama rays: its
+// angles reach pi, the frustum's stay below pi/4).  In the fast flavour both are the same code.
+BT_DEV void camera_sincos(bool pano, float x, float* sn, float* cs) {
+#ifdef BT_EXACT_SCAN
+    if (!pano) return sincosf(x, sn, cs);
+#endif
+    (void)pano;
+    sincos_poly(x, sn, cs);
+}
+// (sub_i, sub_j): the sub-pixel of this path, i fastest (mod.rs:70-106).
+// Both projections turn the jittered (u, v) into two angles and need one sin / cos of each (one camera_sincos pair, shared):
+//  * PROJ_PERSPECTIVE (the reference): yrot / 2 = xfov * 0.5 * -u * 0.5, xrot / 2 = yfov * 0.5 * -v * 0.5, then the quaternion;
+//  * PROJ_EQUIRECTANGULAR (extension, DESIGN.md §3.6): phi = fl(PI_F * fl(u + pixel_width * 0.5)) and
+//    theta = fl(-PI_F/2 * fl(v + pixel_height * 0.5)) -- pixel (x, y) with zero jitter looks at the centre of texel (x, y) of a
+//    W x H environment map -- and dir_cam = (fl(cos theta * sin phi), sin theta, -fl(cos theta * cos phi)).  Every product and
+//    sum is rounded on its own (x*_rn) and sin / cos come from sincos_poly, so the direction is the oracle's bit for bit in
+//    the exact flavour (in the fast one the jitter's FMA contraction can move u, v by an ulp).  The projection is uniform per call.  An equirectangular camera has has_focus = 0 (make_camera_block): no disk draws.
 BT_DEV void camera_ray(const CameraBlock& cam, const Consts& k, Rng& rng, uint32_t x, uint32_t y, uint32_t sub_i, uint32_t sub_j,
                        V3& origin, V3& direction) {
     float v = (float)y * cam.pixel_height - 1.0f;
@@ -936,7 +953,19 @@ BT_DEV void camera_ray(const CameraBlock& cam, const Consts& k, Rng& rng, uint32
     float v_offset = v_sub * cam.pixel_height + uniform_f32(rng, cam.sv_low, cam.sv_scale);
     u = u + u_offset;
     v = v + v_offset;
-    V3 dir_cam = with_frustum_dir(cam.yfov, cam.xfov, u, v);
+    const bool pano = cam.projection == PROJ_EQUIRECTANGULAR;
+    float a, b;  // (yrot / 2, xrot / 2) or (phi, theta)
+    if (pano) {
+        a = __fmul_rn(3.14159274101257324f, __fadd_rn(u, __fmul_rn(cam.pixel_width, 0.5f)));
+        b = __fmul_rn(-1.57079637050628662f, __fadd_rn(v, __fmul_rn(cam.pixel_height, 0.5f)));
+    } else {
+        a = cam.xfov * 0.5f * -u * 0.5f;
+        b = cam.yfov * 0.5f * -v * 0.5f;
+    }
+    float sa, ca, sb, cb;
+    camera_sincos(pano, a, &sa, &ca);
+    camera_sincos(pano, b, &sb, &cb);
+    V3 dir_cam = pano ? v3(__fmul_rn(cb, sa), sb, -__fmul_rn(cb, ca)) : with_frustum_dir(sa, ca, sb, cb);
     V3 c0 = v3(cam.m[0], cam.m[1], cam.m[2]), c1 = v3(cam.m[3], cam.m[4], cam.m[5]), c2 = v3(cam.m[6], cam.m[7], cam.m[8]);
     V3 t = v3(cam.t[0], cam.t[1], cam.t[2]);
     V3 o = t + v3(0.0f, 0.0f, 0.0f);

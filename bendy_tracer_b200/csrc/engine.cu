@@ -657,6 +657,18 @@ int bt_scene_set_camera_aspect(bt_scene* scene, uint64_t camera_ref, float aspec
     GUARD_END
 }
 
+int bt_scene_set_camera_projection(bt_scene* scene, uint64_t camera_ref, int projection) {
+    if (!scene) return fail(BT_ERR_INVALID_ARG, "NULL argument");
+    GUARD_BEGIN
+    Object& o = scene->scene.get_object(camera_ref);
+    if (o.kind != OBJ_CAMERA) return fail(BT_ERR_SCENE, "called `Option::unwrap()` on a `None` value (object is not a camera)");
+    if (projection != BT_PROJECTION_PERSPECTIVE && projection != BT_PROJECTION_EQUIRECTANGULAR)
+        return fail(BT_ERR_INVALID_ARG, "projection must be BT_PROJECTION_PERSPECTIVE or BT_PROJECTION_EQUIRECTANGULAR");
+    o.camera.projection = projection == BT_PROJECTION_EQUIRECTANGULAR ? PROJ_EQUIRECTANGULAR : PROJ_PERSPECTIVE;  // read per call, like the aspect
+    return BT_OK;
+    GUARD_END
+}
+
 int bt_scene_apply_transform(bt_scene* scene, uint64_t object_ref, const float affine[12]) {
     if (!scene || !affine) return fail(BT_ERR_INVALID_ARG, "NULL argument");
     GUARD_BEGIN

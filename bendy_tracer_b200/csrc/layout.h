@@ -113,6 +113,8 @@ struct SceneHeader {
     int32_t far_prim[2];
 };
 
+enum { PROJ_PERSPECTIVE = 0, PROJ_EQUIRECTANGULAR = 1 };  // BT_PROJECTION_* (bt_scene_set_camera_projection)
+
 struct CameraBlock {                 // reference src/tracer/mod.rs:244-267 hoisted per render call
     float m[9];                      // transform_world matrix3 columns
     float t[3];
@@ -120,6 +122,7 @@ struct CameraBlock {                 // reference src/tracer/mod.rs:244-267 hois
     float su_low, su_scale, sv_low, sv_scale;   // Uniform::from(min..max) for the jitter
     float sub_width;                 // 1/n, 0 for Subsample::None
     uint32_t sub_n;                  // n (1 for None)
+    uint32_t projection;             // PROJ_*; an equirectangular camera is a pinhole (has_focus = 0)
     uint32_t has_focus;
     float focus, aperture;
     float disk_x[3], disk_y[3];      // UnitDisk::new(NEG_Z) basis

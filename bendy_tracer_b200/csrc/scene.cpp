@@ -1681,7 +1681,8 @@ CameraBlock make_camera_block(const Scene& scene, uint64_t camera_ref, uint32_t 
     c.sv_scale = uniform_scale(c.sv_low, 0.5f * c.pixel_height * subpixel_scale);
     c.sub_width = subsample == 0 ? 0.0f : 1.0f / (float)subsample;
     c.sub_n = subsample == 0 ? 1u : subsample;
-    c.has_focus = cam.has_focus ? 1u : 0u;
+    c.projection = cam.projection;
+    c.has_focus = cam.has_focus && cam.projection == PROJ_PERSPECTIVE ? 1u : 0u;  // a panorama is a pinhole
     c.focus = cam.focus;
     c.aperture = 0.5f * cam.focal_length / cam.fstop;  // mod.rs:289
     // UnitDisk::new(Vec3::NEG_Z): any_orthonormal_pair((0,0,-1)) = ((1,-0,0),(0,-1,-0))

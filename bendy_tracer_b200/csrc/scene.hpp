@@ -39,6 +39,7 @@ struct Camera {  // reference src/scene/object/camera.rs:3-10
     float sensor_size, focal_length, aspect_ratio, fstop;
     bool has_focus;
     float focus;
+    uint32_t projection;  // PROJ_* (bt_scene_set_camera_projection): host-only, not part of the wire format
 };
 enum ObjectKind { OBJ_EMPTY, OBJ_CAMERA, OBJ_SPHERE, OBJ_RECT, OBJ_CUBOID };
 

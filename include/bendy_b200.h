@@ -151,6 +151,23 @@ int bt_scene_find_by_tag(const bt_scene* scene, const char* tag, uint64_t* objec
 /* The one scene update main issues: camera.aspect_ratio = w/h through an UpdateQueue
  * (reference src/main.rs:218-223, 337-350). */
 int bt_scene_set_camera_aspect(bt_scene* scene, uint64_t camera_ref, float aspect_ratio);
+/* Camera projection (extension; DESIGN.md §3.6).  PERSPECTIVE (the default) is the reference's frustum.  EQUIRECTANGULAR
+ * renders the whole sphere around the camera in the environment map's convention (bt_scene_set_environment), so a panorama
+ * of an empty scene reproduces its map: with the jittered NDC u, v formed as for PERSPECTIVE (the same two draws and
+ * sub-pixel offsets), u' = u + pixel_width / 2, v' = v + pixel_height / 2 (pixel_width = 2 / width, ...),
+ * phi = PI_F * u', theta = -(PI_F / 2) * v', and the camera-space direction is
+ * (cos theta * sin phi, sin theta, -(cos theta * cos phi)), each product and sum rounded on its own and sin / cos from the
+ * engine's own polynomial in both arithmetic flavours (DESIGN.md §3.6 spells out the order): pixel (x, y) with zero
+ * jitter looks at the centre of texel (x, y) of a width x height map, the centre column along camera -z, columns towards
+ * camera +x, row 0 at the +y pole.  Directions past a pole (sub-pixel offsets on the last row) are used as computed.  The
+ * direction then goes through the camera's world transform as for PERSPECTIVE and the origin is the camera's position.
+ * An equirectangular camera is a pinhole: focus and fstop are ignored and no unit-disk numbers are drawn, so every path
+ * draws exactly two numbers for its camera ray.  sensor_size, focal_length and aspect_ratio do not apply; any width x height
+ * is allowed (width = 2 height gives square pixels).  Host-only: read per render call, never re-flattens or uploads, and
+ * not part of the wire format (bt_scene_to_json is unchanged).  BT_ERR_SCENE for a reference that is not a camera,
+ * BT_ERR_INVALID_ARG for an unknown projection (scene unchanged). */
+enum { BT_PROJECTION_PERSPECTIVE = 0, BT_PROJECTION_EQUIRECTANGULAR = 1 };
+int bt_scene_set_camera_projection(bt_scene* scene, uint64_t camera_ref, int projection);
 /* Object::apply_transform on one object followed by UpdateQueue::commit (reference
  * src/scene/object/mod.rs:212-223, src/scene/mod.rs:204-213): local = local * affine, world and
  * the children's parent transforms are re-derived, device buffers are re-flattened lazily. */
