@@ -14,6 +14,8 @@
  *   - Object iteration order: ascending ObjectRef instead of hashbrown's per-process order.
  *   - Lensing (geodesic segments) exists only when lenses are set; with none the code path is
  *     the reference's try_hit.
+ *   - The environment map and the equirectangular camera exist only when set; with neither the
+ *     code paths are the reference's sample_root and camera_ray.
  */
 #include "bendy_oracle.h"
 
@@ -317,6 +319,9 @@ struct Scene {
     uint64_t root_material;
     std::vector<Lens> lenses;
     orc_lens_config lens_cfg;
+    std::vector<float> env_rgb;          // environment map: env_w * env_h RGB texels, row 0 = +y pole
+    uint32_t env_w = 0, env_h = 0;       // env_w == 0: no map
+    std::map<uint64_t, int> projection;  // camera object_ref -> ORC_PROJECTION_*, only for cameras that are not PERSPECTIVE
 
     const orc_object& get_object(uint64_t r) const {  // src/scene/mod.rs:131-133
         std::map<uint64_t, int>::const_iterator it = object_index.find(r);
@@ -865,6 +870,58 @@ Segment<T> trace_segment(const Scene& scene, const Field<T>& f, const Ray<T>& ra
 }
 
 // ------------------------------------------------------------------------------------------
+// environment map + equirectangular camera (NOT in the reference; DESIGN.md §3.5, §3.6)
+// ------------------------------------------------------------------------------------------
+// Earlier revisions' test layers #include this file and define sincos_poly, equirect_dir and
+// orc_env_lookup themselves: the names here differ so that their tests still build against it.
+// The lookup of device.cuh (env_lookup), operation for operation: every product and sum rounded
+// on its own (-ffp-contract=off), atan2 / sqrt from libm.  Any d, NaN included, reads a texel.
+V3f env_lookup(const float* rgb, uint32_t w, uint32_t h, V3f d) {
+    const float phi = std::atan2(d.x, -d.z), theta = std::atan2(d.y, std::sqrt(d.x * d.x + d.z * d.z));
+    const float u = 0.5f + phi * 0.159154943091895335769f, v = 0.5f - theta * 0.318309886183790671538f;  // 1/(2 pi), 1/pi
+    const float x = std::fmin(std::fmax(u * (float)w - 0.5f, -1.0f), (float)w);
+    const float y = std::fmin(std::fmax(v * (float)h - 0.5f, -1.0f), (float)h);
+    const float fx = std::floor(x), fy = std::floor(y), tx = x - fx, ty = y - fy;
+    const uint32_t c0 = fx < 0.0f ? w - 1 : std::min((uint32_t)fx, w - 1), c1 = c0 + 1 == w ? 0 : c0 + 1;
+    const uint32_t r0 = fy < 0.0f ? 0 : std::min((uint32_t)fy, h - 1), r1 = fy < 0.0f ? 0 : std::min((uint32_t)fy + 1, h - 1);
+    const float *a = rgb + 3 * ((size_t)r0 * w + c0), *b = rgb + 3 * ((size_t)r0 * w + c1);
+    const float *c = rgb + 3 * ((size_t)r1 * w + c0), *e = rgb + 3 * ((size_t)r1 * w + c1);
+    float out[3];
+    for (int k = 0; k < 3; ++k) out[k] = lerp(lerp(a[k], b[k], tx), lerp(c[k], e[k], tx), ty);
+    return mk<float>(out[0], out[1], out[2]);
+}
+
+// device.cuh's sincos_poly, operation for operation: Cody-Waite reduction by pi/2 and the Cephes polynomials in explicit FMAs
+void panorama_sincos(float x, float* sn, float* cs) {
+    const float k = std::rint(x * 0.636619772367581343f);
+    float y = std::fma(k, -1.5703125f, x);
+    y = std::fma(k, -4.837512969970703125e-4f, y);
+    y = std::fma(k, -7.549789954891882e-8f, y);
+    const int q = (int)k;
+    const float y2 = y * y;
+    float s = std::fma(-1.9515295891e-4f, y2, 8.3321608736e-3f);
+    s = std::fma(s, y2, -1.6666654611e-1f);
+    s = std::fma(s * y2, y, y);
+    float c = std::fma(2.443315711809948e-5f, y2, -1.388731625493765e-3f);
+    c = std::fma(c, y2, 4.166664568298827e-2f);
+    c = std::fma(c * y2, y2, std::fma(-0.5f, y2, 1.0f));
+    const float a = (q & 1) ? c : s, b = (q & 1) ? s : c;
+    *sn = (q & 2) ? -a : a;
+    *cs = ((q + 1) & 2) ? -b : b;
+}
+
+// device.cuh camera_ray's equirectangular branch, operation for operation: the camera-space
+// direction for the jittered NDC (u, v) before the half-pixel offset
+V3f panorama_dir(float u, float v, float pixel_width, float pixel_height) {
+    const float phi = 3.14159274101257324f * (u + pixel_width * 0.5f);
+    const float theta = -1.57079637050628662f * (v + pixel_height * 0.5f);
+    float sp, cp, st, ct;
+    panorama_sincos(phi, &sp, &cp);
+    panorama_sincos(theta, &st, &ct);
+    return mk<float>(ct * sp, st, -(ct * cp));
+}
+
+// ------------------------------------------------------------------------------------------
 // tracer  (src/tracer/mod.rs)
 // ------------------------------------------------------------------------------------------
 struct ChunkConfig {  // mod.rs:205-230
@@ -1032,7 +1089,7 @@ struct ChunkState {
         return found;
     }
 
-    // mod.rs:429-452
+    // mod.rs:429-452 (+ the environment map's factor in the escape direction when the scene has a map)
     ColorData sample_root(const Rayf& ray) {
         const Data& d = scene->get_material(scene->root_material, "expected root material to be a material");
         Manifold<float> manifold;
@@ -1049,6 +1106,7 @@ struct ChunkState {
         ShaderData data = shade(d.d, manifold, clip());
         ColorData cd = data.has_albedo ? data.albedo : ColorData();
         cd.color = cd.color + e;
+        if (scene->env_w != 0) cd.color = cd.color * env_lookup(scene->env_rgb.data(), scene->env_w, scene->env_h, ray.direction);
         return cd;
     }
 
@@ -1178,6 +1236,7 @@ struct CameraSetup {
     Basis defocus_basis;
     uint32_t sub_n;  // 1 for Subsample::None
     float sub_width;
+    int projection;  // ORC_PROJECTION_*
     CameraSetup() : defocus_basis(mk<float>(0.0f, 0.0f, -1.0f)) {}
 };
 
@@ -1197,10 +1256,13 @@ CameraSetup camera_setup(const Scene& scene, uint64_t camera_ref, const ChunkCon
     cs.scatter_v = UniformF32::make(-0.5f * cs.pixel_height * subpixel_scale, 0.5f * cs.pixel_height * subpixel_scale);
     cs.sub_n = cfg.subsample == 0 ? 1 : cfg.subsample;
     cs.sub_width = cfg.subsample == 0 ? 0.0f : 1.0f / (float)cfg.subsample;
+    std::map<uint64_t, int>::const_iterator p = scene.projection.find(camera_ref);
+    cs.projection = p == scene.projection.end() ? ORC_PROJECTION_PERSPECTIVE : p->second;
     return cs;
 }
 
-// mod.rs:272-302: one camera ray; draws jitter-u, jitter-v, [disk angle, disk radius]
+// mod.rs:272-302: one camera ray; draws jitter-u, jitter-v, [disk angle, disk radius].
+// The equirectangular camera forms (u, v) the same way and is a pinhole: no disk draws.
 Rayf camera_ray(const CameraSetup& cs, Rng& rng, uint32_t x, uint32_t y, uint32_t sub_index) {
     float v = (float)y * cs.pixel_height - 1.0f;
     float u = (float)x * cs.pixel_width - 1.0f;
@@ -1214,6 +1276,12 @@ Rayf camera_ray(const CameraSetup& cs, Rng& rng, uint32_t x, uint32_t y, uint32_
     float v_offset = v_sub * cs.pixel_height + cs.scatter_v.sample(rng);
     u = u + u_offset;
     v = v + v_offset;
+    if (cs.projection == ORC_PROJECTION_EQUIRECTANGULAR) {
+        const V3f dir_cam = panorama_dir(u, v, cs.pixel_width, cs.pixel_height);
+        V3f origin = cs.tf.translation + mk<float>(0, 0, 0);  // Affine3A * Ray, ray.rs:126-137
+        V3f direction = normalize_or_zero_s(transform_vector(cs.tf, dir_cam));
+        return ray_new(origin, direction);
+    }
     Rayf ray;
     ray.origin = mk<float>(0, 0, 0);
     ray.direction = with_frustum_dir(cs.yfov, cs.xfov, u, v);
@@ -1286,6 +1354,35 @@ int orc_scene_set_camera_aspect(void* scene, uint64_t camera_ref, float aspect) 
         return -1;
     }
     s->objects[it->second].aspect_ratio = aspect;
+    return 0;
+}
+
+int orc_scene_set_environment(void* scene, const float* rgb, uint32_t width, uint32_t height) {
+    Scene* s = (Scene*)scene;
+    if (!rgb || width == 0 || height == 0) {
+        s->env_rgb.clear();
+        s->env_w = s->env_h = 0;
+        return 0;
+    }
+    s->env_rgb.assign(rgb, rgb + (size_t)width * height * 3);
+    s->env_w = width;
+    s->env_h = height;
+    return 0;
+}
+
+int orc_scene_set_camera_projection(void* scene, uint64_t camera_ref, int projection) {
+    Scene* s = (Scene*)scene;
+    std::map<uint64_t, int>::iterator it = s->object_index.find(camera_ref);
+    if (it == s->object_index.end() || s->objects[it->second].kind != ORC_CAMERA) {
+        g_last_error = g_last_error_shared = "expected a camera object";
+        return -1;
+    }
+    if (projection != ORC_PROJECTION_PERSPECTIVE && projection != ORC_PROJECTION_EQUIRECTANGULAR) {
+        g_last_error = g_last_error_shared = "unknown projection";
+        return -1;
+    }
+    if (projection == ORC_PROJECTION_PERSPECTIVE) s->projection.erase(camera_ref);
+    else s->projection[camera_ref] = projection;
     return 0;
 }
 
@@ -1559,6 +1656,14 @@ int orc_uniform_usize(uint64_t seed, uint64_t n_range, uint64_t* out, int n) {
 void orc_with_frustum(float yfov, float xfov, float u, float v, float dir_out[3]) {
     V3f d = with_frustum_dir(yfov, xfov, u, v);
     dir_out[0] = d.x; dir_out[1] = d.y; dir_out[2] = d.z;
+}
+void orc_environment_lookup(const float* rgb, uint32_t width, uint32_t height, const float d[3], float out[3]) {
+    V3f c = env_lookup(rgb, width, height, mk<float>(d[0], d[1], d[2]));
+    out[0] = c.x; out[1] = c.y; out[2] = c.z;
+}
+void orc_equirect_dir(float u, float v, float pixel_width, float pixel_height, float out[3]) {
+    V3f d = panorama_dir(u, v, pixel_width, pixel_height);
+    out[0] = d.x; out[1] = d.y; out[2] = d.z;
 }
 void orc_any_orthonormal_pair(const float n[3], float a_out[3], float b_out[3]) {
     V3f a, b;

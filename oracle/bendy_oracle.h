@@ -32,6 +32,8 @@ enum { ORC_CS_NONE = 0, ORC_CS_NORMAL = 1, ORC_CS_LINEAR = 2, ORC_CS_SRGB = 3 };
 /* Face, reference src/tracer/ray.rs:8-15 (+ miss / capture codes used by the probe) */
 enum { ORC_FACE_FRONT = 0, ORC_FACE_BACK = 1, ORC_FACE_VOLUME = 2, ORC_FACE_VOLUME_FRONT = 3,
        ORC_FACE_VOLUME_BACK = 4, ORC_FACE_MISS = -1, ORC_FACE_CAPTURED = -2 };
+/* camera projection extension (NOT in the reference): the engine's BT_PROJECTION_* values */
+enum { ORC_PROJECTION_PERSPECTIVE = 0, ORC_PROJECTION_EQUIRECTANGULAR = 1 };
 
 typedef struct {            /* Rect, reference src/scene/object/rect.rs:11-19 */
     uint64_t material;
@@ -102,6 +104,13 @@ void* orc_scene_create(const orc_object* objects, int n_objects, const orc_data*
                        uint64_t root_material);
 void orc_scene_set_lenses(void* scene, const float* xyzr, int n, const orc_lens_config* cfg);
 int orc_scene_set_camera_aspect(void* scene, uint64_t camera_ref, float aspect);
+/* environment map extension (NOT in the reference; DESIGN.md §3.5): width * height RGB texels,
+ * row 0 = +y pole, copied; rgb = NULL or a zero size clears the map.  Returns 0. */
+int orc_scene_set_environment(void* scene, const float* rgb, uint32_t width, uint32_t height);
+/* camera projection extension (NOT in the reference; DESIGN.md §3.6): ORC_PROJECTION_*.
+ * returns 0, or -1 (message via orc_last_error, scene unchanged) for a reference that is not a
+ * camera or an unknown projection */
+int orc_scene_set_camera_projection(void* scene, uint64_t camera_ref, int projection);
 void orc_scene_destroy(void* scene);
 
 /* Tracer::render (src/tracer/mod.rs:179-202) with the keyed RNG stream of DESIGN.md.
@@ -135,6 +144,10 @@ void orc_standard_f32(uint64_t seed, float* out, int n);
 int orc_gen_bool(uint64_t seed, double p, uint8_t* out, int n);
 int orc_uniform_usize(uint64_t seed, uint64_t n_range, uint64_t* out, int n);
 void orc_with_frustum(float yfov, float xfov, float u, float v, float dir_out[3]);
+/* the environment map's factor for one direction (any d: non-unit, zero, NaN / inf components) */
+void orc_environment_lookup(const float* rgb, uint32_t width, uint32_t height, const float d[3], float out[3]);
+/* the equirectangular camera-space direction for the NDC (u, v) before the half-pixel offset */
+void orc_equirect_dir(float u, float v, float pixel_width, float pixel_height, float out[3]);
 void orc_any_orthonormal_pair(const float n[3], float a_out[3], float b_out[3]);
 void orc_distr(int which /*0 sphere,1 hemisphere,2 cosine,3 disk*/, uint64_t seed, const float n[3],
                float* out, int count);

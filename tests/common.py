@@ -10,8 +10,9 @@ LENS_SCENE = np.array([[1.362, 1.577, 6.114, 0.2]], np.float32)
 LENS_VOLUME = np.array([[2.4 - 6 * 0.1705, 2.7 - 6 * 0.1908, 12.0 - 6 * 0.9667, 0.2]], np.float32)
 
 
-def load_pair(name, width, height, lenses=None):
-    """(oracle scene, engine scene, camera ref) with camera.aspect_ratio = width / height (main.rs:218-223)"""
+def load_pair(name, width, height, lenses=None, projection=None):
+    """(oracle scene, engine scene, camera ref) with camera.aspect_ratio = width / height (main.rs:218-223), and the
+    lenses and the camera projection, when given, set on both"""
     import bendy_tracer_b200 as bt
     path = O.scene_path(name)
     osc = O.OracleScene.load(path)
@@ -24,6 +25,9 @@ def load_pair(name, width, height, lenses=None):
     if lenses is not None:
         osc.set_lenses(lenses)
         esc.set_lenses(lenses)
+    if projection is not None:
+        osc.set_projection(cam, projection)
+        esc.set_camera_projection(cam, projection)
     return osc, esc, cam
 
 

@@ -20,6 +20,7 @@ FLAT, DIFFUSE, METALLIC, GLASS, EMISSIVE = range(5)
 OUT_FULL, OUT_ALBEDO, OUT_NORMAL, OUT_DEPTH = range(4)
 CS_NONE, CS_NORMAL, CS_LINEAR, CS_SRGB = range(4)
 FACE_MISS, FACE_CAPTURED = -1, -2
+PERSPECTIVE, EQUIRECTANGULAR = 0, 1
 
 
 class OrcRect(C.Structure):
@@ -76,14 +77,14 @@ def lib():
     global _lib
     if _lib is not None:
         return _lib
-    path = os.path.join(ORACLE_DIR, "libbendy_oracle.so")
-    if not os.path.exists(path):
-        build()
-    L = C.CDLL(path)
+    build()                                      # make: rebuilds a library older than its sources, else a no-op
+    L = C.CDLL(os.path.join(ORACLE_DIR, "libbendy_oracle.so"))
     L.orc_scene_create.restype = C.c_void_p
     L.orc_scene_create.argtypes = [C.POINTER(OrcObject), C.c_int, C.POINTER(OrcData), C.c_int, C.c_uint64]
     L.orc_scene_set_lenses.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(OrcLensConfig)]
     L.orc_scene_set_camera_aspect.argtypes = [C.c_void_p, C.c_uint64, C.c_float]
+    L.orc_scene_set_environment.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32]
+    L.orc_scene_set_camera_projection.argtypes = [C.c_void_p, C.c_uint64, C.c_int]
     L.orc_scene_destroy.argtypes = [C.c_void_p]
     L.orc_render.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(OrcConfig), C.c_uint64, C.c_uint64,
                              C.c_void_p, C.c_uint32, C.c_uint32, C.c_int, C.POINTER(C.c_uint64)]
@@ -105,6 +106,8 @@ def lib():
     L.orc_gen_bool.argtypes = [C.c_uint64, C.c_double, C.c_void_p, C.c_int]
     L.orc_uniform_usize.argtypes = [C.c_uint64, C.c_uint64, C.c_void_p, C.c_int]
     L.orc_with_frustum.argtypes = [C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]
+    L.orc_environment_lookup.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p]
+    L.orc_equirect_dir.argtypes = [C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]
     L.orc_any_orthonormal_pair.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.orc_distr.argtypes = [C.c_int, C.c_uint64, C.c_void_p, C.c_void_p, C.c_int]
     L.orc_sphere_hit.argtypes = [C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_float, C.c_float,
@@ -265,6 +268,20 @@ class OracleScene:
         self.lenses = xyzr
         lib().orc_scene_set_lenses(self.handle, _p(xyzr), len(xyzr), C.byref(c))
 
+    def set_environment(self, rgb):
+        """(H, W, 3) RGB, row 0 = +y pole, centre column along -z; None clears it"""
+        if rgb is None:
+            lib().orc_scene_set_environment(self.handle, None, 0, 0)
+            return
+        rgb = np.ascontiguousarray(rgb, np.float32)
+        h, w, _ = rgb.shape
+        lib().orc_scene_set_environment(self.handle, _p(rgb), w, h)
+
+    def set_projection(self, camera_ref, projection):
+        """PERSPECTIVE or EQUIRECTANGULAR"""
+        if lib().orc_scene_set_camera_projection(self.handle, camera_ref, int(projection)) != 0:
+            raise OraclePanic(lib().orc_last_error().decode())
+
     def render(self, camera_ref, cfg, width, height, seed=0, sample_base=0, buffer=None, n_threads=None):
         """Tracer::render into an RGBA32F buffer (alpha 1, as Buffer::new). Returns (buffer, samples, status)."""
         if buffer is None:
@@ -310,6 +327,25 @@ def resolve_u8(buffer, samples, color_space):
     h, w, _ = buffer.shape
     out = np.zeros((h, w, 4), np.uint8)
     lib().orc_resolve_u8(_p(np.ascontiguousarray(buffer, np.float32)), w, h, samples, color_space, _p(out))
+    return out
+
+
+def env_lookup(rgb, d):
+    """the map's factor for direction(s) d ((3,) or (n, 3)) in the (H, W, 3) map rgb"""
+    rgb = np.ascontiguousarray(rgb, np.float32)
+    h, w, _ = rgb.shape
+    d = np.ascontiguousarray(d, np.float32)
+    flat = d.reshape(-1, 3)
+    out = np.zeros_like(flat)
+    for i in range(len(flat)):
+        lib().orc_environment_lookup(_p(rgb), w, h, _p(flat[i]), _p(out[i]))
+    return out.reshape(d.shape)
+
+
+def equirect_dir(u, v, pixel_width, pixel_height):
+    """camera-space direction of an equirectangular camera for the NDC (u, v) before the half-pixel offset"""
+    out = np.zeros(3, np.float32)
+    lib().orc_equirect_dir(u, v, pixel_width, pixel_height, _p(out))
     return out
 
 

@@ -1,8 +1,8 @@
 """The environment map (bt_scene_set_environment / Scene.set_environment) on the host: the lookup's known answers in the
 oracle, the Einstein ring it makes visible under a lens, the API's argument checks and the CLI's PFM reader.
 
-The oracle side is tests/oracle_env.cpp: the unchanged CPU oracle with the map multiplied into sample_root.
-Semantics (DESIGN.md §3.5): an escaping path's colour is sample_root's colour times the bilinear lookup of
+The oracle side is oracle/bendy_oracle.cpp with a map set (OracleScene.set_environment): its sample_root multiplies the
+colour by the map's lookup.  Semantics (DESIGN.md §3.5): an escaping path's colour is sample_root's colour times the bilinear lookup of
 an equirectangular map in its escape direction; row 0 is the +y pole, the centre column looks along -z."""
 import ctypes as C
 import json
@@ -15,9 +15,7 @@ import pytest
 import bendy_tracer_b200 as bt
 import oracle_ffi as O
 from bendy_tracer_b200 import _ffi
-import oracle_env as OE
-from common import LENS_SCENE, LENS_VOLUME, oracle_render
-from oracle_env import load_pair
+from common import LENS_SCENE, LENS_VOLUME, load_pair, oracle_render
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CLI = os.path.join(ROOT, "bendy_tracer_b200", "csrc", "bendy_b200_cli")
@@ -45,7 +43,7 @@ def test_texel_centre_returns_the_texel():
     env = random_map(h, w, 1)
     for r in range(h):
         for c in range(0, w, 3):
-            got = OE.env_lookup(env, texel_dir(r, c, h, w))
+            got = O.env_lookup(env, texel_dir(r, c, h, w))
             assert np.allclose(got, env[r, c], atol=2e-5), (r, c)
 
 
@@ -53,17 +51,17 @@ def test_forward_direction_is_the_map_centre():
     """d = (0, 0, -1): u = v = 0.5, i.e. the corner shared by the four central texels of an even-sized map"""
     h, w = 8, 12
     env = random_map(h, w, 2)
-    got = OE.env_lookup(env, [0.0, 0.0, -1.0])
+    got = O.env_lookup(env, [0.0, 0.0, -1.0])
     r, c = h // 2 - 1, w // 2 - 1
     want = lerp(lerp(env[r, c], env[r, c + 1], 0.5), lerp(env[r + 1, c], env[r + 1, c + 1], 0.5), 0.5)
     assert np.array_equal(got, want)
     # odd-sized: the centre texel exactly
     env = random_map(7, 9, 3)
-    assert np.array_equal(OE.env_lookup(env, [0.0, 0.0, -1.0]), env[3, 4])
+    assert np.array_equal(O.env_lookup(env, [0.0, 0.0, -1.0]), env[3, 4])
     # +x is a quarter turn right of the centre column (x = 0.75 W - 0.5), -x a quarter turn left, +z the seam
-    assert np.allclose(OE.env_lookup(env, [1.0, 0.0, 0.0]), lerp(env[3, 6], env[3, 7], 0.25), atol=1e-5)
-    assert np.allclose(OE.env_lookup(env, [-1.0, 0.0, 0.0]), lerp(env[3, 1], env[3, 2], 0.75), atol=1e-5)
-    assert np.allclose(OE.env_lookup(env, [0.0, 0.0, 1.0]), lerp(env[3, 8], env[3, 0], 0.5), atol=1e-5)
+    assert np.allclose(O.env_lookup(env, [1.0, 0.0, 0.0]), lerp(env[3, 6], env[3, 7], 0.25), atol=1e-5)
+    assert np.allclose(O.env_lookup(env, [-1.0, 0.0, 0.0]), lerp(env[3, 1], env[3, 2], 0.75), atol=1e-5)
+    assert np.allclose(O.env_lookup(env, [0.0, 0.0, 1.0]), lerp(env[3, 8], env[3, 0], 0.5), atol=1e-5)
 
 
 def test_poles_reach_the_first_and_last_rows():
@@ -72,9 +70,9 @@ def test_poles_reach_the_first_and_last_rows():
     env[0] = [0.25, 0.5, 0.75]
     env[-1] = [1.0, 2.0, 3.0]
     for d in ([0, 1, 0], [0.0, 1.0, 1e-4], [0.01, 1.0, -0.01], [-0.03, 1.0, 0.02]):
-        assert np.array_equal(OE.env_lookup(env, d), env[0, 0]), d
+        assert np.array_equal(O.env_lookup(env, d), env[0, 0]), d
     for d in ([0, -1, 0], [0.0, -1.0, 1e-4], [0.02, -1.0, 0.01]):
-        assert np.array_equal(OE.env_lookup(env, d), env[-1, 0]), d
+        assert np.array_equal(O.env_lookup(env, d), env[-1, 0]), d
 
 
 def test_seam_is_continuous():
@@ -83,14 +81,14 @@ def test_seam_is_continuous():
     env = random_map(h, w, 5)
     for eps in (1e-2, 1e-3, 1e-4):
         for theta in (-0.7, 0.0, 0.3, 1.2):
-            a = OE.env_lookup(env, [np.cos(theta) * np.sin(np.pi - eps), np.sin(theta), -np.cos(theta) * np.cos(np.pi - eps)])
-            b = OE.env_lookup(env, [np.cos(theta) * np.sin(-np.pi + eps), np.sin(theta), -np.cos(theta) * np.cos(-np.pi + eps)])
+            a = O.env_lookup(env, [np.cos(theta) * np.sin(np.pi - eps), np.sin(theta), -np.cos(theta) * np.cos(np.pi - eps)])
+            b = O.env_lookup(env, [np.cos(theta) * np.sin(-np.pi + eps), np.sin(theta), -np.cos(theta) * np.cos(-np.pi + eps)])
             assert np.abs(a - b).max() <= 2 * eps / (2 * np.pi) * w + 1e-5, (eps, theta, a, b)
     # exactly on the seam: the midpoint of the last and the first column
     r = 5
     d = texel_dir(r, 0, h, w)
     d = np.array([0.0, d[1], np.cos(np.arcsin(d[1]))])
-    assert np.allclose(OE.env_lookup(env, d), lerp(env[r, -1], env[r, 0], 0.5), atol=1e-5)
+    assert np.allclose(O.env_lookup(env, d), lerp(env[r, -1], env[r, 0], 0.5), atol=1e-5)
 
 
 def test_bilinear_midpoint_is_the_average():
@@ -101,7 +99,7 @@ def test_bilinear_midpoint_is_the_average():
         theta = (0.5 - (r + 1) / h) * np.pi
         d = [np.cos(theta) * np.sin(phi), np.sin(theta), -np.cos(theta) * np.cos(phi)]
         want = (env[r, c] + env[r, c + 1] + env[r + 1, c] + env[r + 1, c + 1]) / 4
-        assert np.allclose(OE.env_lookup(env, d), want, atol=2e-5), (r, c)
+        assert np.allclose(O.env_lookup(env, d), want, atol=2e-5), (r, c)
 
 
 @pytest.mark.parametrize("h,w", [(1, 1), (1, 3), (2, 1), (5, 7), (64, 128)])
@@ -113,31 +111,18 @@ def test_any_direction_returns_a_value_of_the_map(h, w):
     rng = np.random.default_rng(8)
     unit = rng.normal(size=(200, 3))
     unit /= np.linalg.norm(unit, axis=1, keepdims=True)
-    base = OE.env_lookup(env, unit)
+    base = O.env_lookup(env, unit)
     for k in (1e-3, 0.37, 1.01, 7.5, 1e3):                        # (not 1e-30 / 1e30: d.x^2 + d.z^2 under- / overflows)
-        assert np.allclose(OE.env_lookup(env, unit * k), base, atol=1e-4), k
+        assert np.allclose(O.env_lookup(env, unit * k), base, atol=1e-4), k
     nan, inf = float("nan"), float("inf")
     odd = [[0, 0, 0], [-0.0, 0.0, -0.0], [nan, nan, nan], [nan, 0, -1], [0, nan, -1], [1, 0, nan], [inf, 0, 0],
            [-inf, inf, 0], [inf, inf, inf], [0, -inf, 0], [nan, inf, -inf], [1e38, 1e38, 1e38], [1e-45, 0, -1e-45],
            [np.nextafter(np.float32(0), np.float32(1)), 0, 0], [0, 0, 1], [-1e-7, 0, 1], [1e-7, 0, 1]]
-    got = OE.env_lookup(env, odd)
+    got = O.env_lookup(env, odd)
     assert np.isfinite(got).all()
     assert ((got >= lo - 1e-6) & (got <= hi + 1e-6)).all()
     texels = {tuple(t) for t in env.reshape(-1, 3)}
     assert tuple(got[2]) in texels                                   # all-NaN: one texel, no blend
-
-
-def test_env_oracle_without_a_map_is_the_oracle():
-    """the oracle library with the map hooked into sample_root renders what oracle/ renders as long as no map is set"""
-    from common import load_pair as plain_pair
-    for name, lens in (("scene", LENS_SCENE), ("cloud", None), ("cornell", None)):
-        w, h = 48, 27
-        env_osc, _, cam = load_pair(name, w, h, lenses=lens)
-        osc = plain_pair(name, w, h, lenses=lens)[0]
-        a = oracle_render(env_osc, cam, w, h, 1, 2, seed=4)[0]
-        assert np.array_equal(a, oracle_render(osc, cam, w, h, 1, 2, seed=4)[0]), name
-        env_osc.set_environment(np.full((2, 3, 3), 0.5, np.float32))
-        assert not np.array_equal(oracle_render(env_osc, cam, w, h, 1, 2, seed=4)[0], a) or name == "cornell"
 
 
 def test_all_ones_map_is_bit_identical_to_no_map():
@@ -223,7 +208,7 @@ def test_einstein_ring():
     assert abs(theta_e - np.sqrt(2 * R_S / D_L)) <= 0.05 * np.sqrt(2 * R_S / D_L), theta_e
 
     size, spp = 192, 4
-    osc = OE.EnvOracleScene(doc)
+    osc = O.OracleScene(doc)
     osc.set_camera_aspect(0, 1.0)
     osc.set_environment(disc_map(fwd))
     cfg = O.make_config(samples=spp)

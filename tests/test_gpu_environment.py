@@ -1,7 +1,7 @@
 """The environment map on the GPU (bt_scene_set_environment / Scene.set_environment): parity with the oracle on identical
 sample sets, bit-identity of an all-ones map with no map in every kernel, pooled = lane kernel with a map, what the map
 must not touch (AOV outputs, work counters) and the plumbing (host buffers, multi-device engines, clear, replacement
-between asynchronous renders, the CLI's PFM reader)."""
+between asynchronous renders, the CLI's PFM reader).  The oracle side is OracleScene with the same map set."""
 import json
 import os
 import subprocess
@@ -9,8 +9,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from common import LENS_SCENE, LENS_VOLUME, SCENES, mae_per_channel, oracle_render, synthetic_scene
-from oracle_env import load_pair
+from common import LENS_SCENE, LENS_VOLUME, SCENES, load_pair, mae_per_channel, oracle_render, synthetic_scene
 
 pytestmark = pytest.mark.gpu
 
@@ -65,9 +64,9 @@ def engine_scene(name, w, h, lens=None, precision=None):
 
 def bvh_pair(w, h):
     import bendy_tracer_b200 as bt
-    from oracle_env import EnvOracleScene
+    import oracle_ffi as O
     doc = synthetic_scene(200, 100, 20, seed=5)
-    osc, esc = EnvOracleScene(doc), bt.Scene.from_json(json.dumps(doc))
+    osc, esc = O.OracleScene(doc), bt.Scene.from_json(json.dumps(doc))
     cam = esc.find_by_tag("camera")
     aspect = float(np.float32(w) / np.float32(h))
     osc.set_camera_aspect(cam, aspect)

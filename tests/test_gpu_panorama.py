@@ -1,7 +1,7 @@
 """The equirectangular camera on the GPU (bt_scene_set_camera_projection / Scene.set_camera_projection): camera-ray and image
 parity with the oracle on identical sample sets, the pooled and lane kernels bit for bit, switching back to the perspective
 camera, the round trip through an environment map, and the plumbing (host buffers, multi-device engines, work counters,
-the CLI)."""
+the CLI).  The oracle side is OracleScene with the same projection and map set (common.load_pair(..., projection=EQ))."""
 import json
 import os
 import subprocess
@@ -9,20 +9,19 @@ import subprocess
 import numpy as np
 import pytest
 
-import oracle_camera as OC
-from common import LENS_SCENE, LENS_VOLUME, mae_per_channel, oracle_render, synthetic_scene
+import oracle_ffi as O
+from common import LENS_SCENE, LENS_VOLUME, load_pair, mae_per_channel, oracle_render, synthetic_scene
 from test_gpu_environment import _read_png, render, smooth_map, write_pfm
 from test_panorama import camera_doc, filtered_map, round_trip_error, rotation
 
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EQ = OC.EQUIRECTANGULAR
+EQ = O.EQUIRECTANGULAR
 
 
 def engine_scene(name, w, h, lens=None, precision=None, projection=EQ):
     import bendy_tracer_b200 as bt
-    import oracle_ffi as O
     sc = bt.Scene.load(O.scene_path(name))
     cam = sc.find_by_tag("camera")
     sc.set_camera_aspect(cam, float(np.float32(w) / np.float32(h)))
@@ -39,7 +38,7 @@ def bvh_pair():
     """synthetic_scene (its camera among the primitives: the panorama sees them in every direction), both sides panoramic"""
     import bendy_tracer_b200 as bt
     doc = synthetic_scene(200, 100, 20, seed=5)
-    osc, esc = OC.CameraOracleScene(doc), bt.Scene.from_json(json.dumps(doc))
+    osc, esc = O.OracleScene(doc), bt.Scene.from_json(json.dumps(doc))
     cam = esc.find_by_tag("camera")
     osc.set_projection(cam, EQ)
     esc.set_camera_projection(cam, EQ)
@@ -55,9 +54,8 @@ def test_camera_rays(precision, subsample):
     """scene.json.gz's camera (it has a focus: a panorama ignores it) at 128 x 64: the exact flavour is the oracle bit for bit,
     the fast one within test_gpu_parity's bar (its jitter's FMA contraction moves u, v by an ulp)"""
     import bendy_tracer_b200 as bt
-    import oracle_ffi as O
     w, h = 128, 64
-    osc, esc, cam = OC.load_pair("scene", w, h)
+    osc, esc, cam = load_pair("scene", w, h, projection=EQ)
     esc.set_precision(precision)
     rng = np.random.default_rng(2)
     n = 8192
@@ -94,7 +92,7 @@ def test_parity_with_oracle(name, lens, env, precision):
     if precision == "fast" and name == "cloud" and lens is not None:
         pytest.skip("the fast stepper through a volume is above the bar with or without a panorama; AUTO renders it exact")
     w, h, passes = 128, 64, 2
-    osc, esc, cam = bvh_pair() if name == "bvh" else OC.load_pair(name, w, h, lenses=lens)
+    osc, esc, cam = bvh_pair() if name == "bvh" else load_pair(name, w, h, lenses=lens, projection=EQ)
     esc.set_precision(precision)
     if precision == "fast" and lens is not None:
         esc.set_lenses(lens, bt.LensConfig(exact_rsqrt=True))
@@ -113,7 +111,7 @@ def test_parity_with_oracle(name, lens, env, precision):
 def test_parity_subsample_none_and_aov_outputs(output):
     """the lensed scene with a map, exact flavour, subsample None, colour and the three AOV outputs"""
     w, h = 128, 64
-    osc, esc, cam = OC.load_pair("scene", w, h, lenses=LENS_SCENE)
+    osc, esc, cam = load_pair("scene", w, h, lenses=LENS_SCENE, projection=EQ)
     esc.set_precision("exact")
     m = smooth_map(32, 64, 4)
     osc.set_environment(m)
@@ -152,7 +150,7 @@ def test_back_to_perspective_is_bit_identical(name, lens, precision):
     ref = render(plain, cam, w, h, 1, 2)
     sc, _ = engine_scene(name, w, h, lens, precision)
     pano = render(sc, cam, w, h, 1, 2)
-    sc.set_camera_projection(cam, OC.PERSPECTIVE)
+    sc.set_camera_projection(cam, O.PERSPECTIVE)
     assert np.array_equal(render(sc, cam, w, h, 1, 2), ref)
     assert not np.array_equal(pano, ref)
 
@@ -238,7 +236,6 @@ def test_render_stats_count_every_path(lens):
 def test_cli_renders_a_panorama(tmp_path):
     """bendy_b200_cli --projection equirectangular --lens --environment renders what the API renders with the same seed"""
     import bendy_tracer_b200 as bt
-    import oracle_ffi as O
     w, h, samples = 128, 64, 8
     env = smooth_map(32, 64, 10)
     env[:8] *= 3.0

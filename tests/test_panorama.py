@@ -3,8 +3,8 @@ known answers in the oracle, the convention shared with the environment map (eve
 panorama of an empty scene reproduces the map, filtered), an Einstein ring in a panorama, the API's argument checks and the
 CLI's --projection.
 
-The oracle side is tests/oracle_camera.cpp: the unchanged CPU oracle with the environment map (oracle_env.cpp) and the
-projection routed into its camera_ray.  Semantics (DESIGN.md §3.6): pixel (x, y) with zero jitter looks at the centre of
+The oracle side is oracle/bendy_oracle.cpp with the camera switched to EQUIRECTANGULAR (OracleScene.set_projection): its
+camera_ray forms the jittered (u, v) as the perspective camera does and turns them into a panorama direction.  Semantics (DESIGN.md §3.6): pixel (x, y) with zero jitter looks at the centre of
 texel (x, y) of a map of the image's size; the centre column looks along camera -z, columns grow towards camera +x, row 0
 is the +y pole; a pinhole."""
 import json
@@ -15,11 +15,9 @@ import numpy as np
 import pytest
 
 import bendy_tracer_b200 as bt
-import oracle_camera as OC
-import oracle_env as OE
 import oracle_ffi as O
 from bendy_tracer_b200 import _ffi
-from common import LENS_SCENE, oracle_render
+from common import LENS_SCENE, load_pair, oracle_render
 from test_environment import DISC, D_L, R_S, disc_map, einstein_angle_f64, ring_scene
 from test_gpu_environment import smooth_map
 
@@ -31,7 +29,7 @@ F = np.float32
 def pixel_dir(x, y, w, h):
     """the oracle's zero-jitter camera-space direction of pixel (x, y), u and v formed in f32 as camera_ray forms them"""
     pw, ph = F(2) * (F(1) / F(w)), F(2) * (F(1) / F(h))
-    return OC.equirect_dir(F(x) * pw - F(1), F(y) * ph - F(1), pw, ph)
+    return O.equirect_dir(F(x) * pw - F(1), F(y) * ph - F(1), pw, ph)
 
 
 def texel_dir(r, c, h, w):
@@ -54,12 +52,12 @@ def test_centre_pixel_looks_forward():
     """odd sizes: the centre pixel's zero-jitter direction is camera -z; the exact NDC origin too, bit for bit"""
     for w, h in ((9, 5), (255, 127)):
         assert np.allclose(pixel_dir(w // 2, h // 2, w, h), [0, 0, -1], atol=1e-6)
-    assert np.array_equal(OC.equirect_dir(F(-0.0625), F(-0.125), F(0.125), F(0.25)), F([0, -0.0, -1]))
+    assert np.array_equal(O.equirect_dir(F(-0.0625), F(-0.125), F(0.125), F(0.25)), F([0, -0.0, -1]))
 
 
 def test_left_edge_looks_backwards():
     """u' = -1: phi = -pi, the direction +z (sin of the rounded pi is 8.7e-8, the azimuth -pi or +pi)"""
-    d = OC.equirect_dir(F(-1.125), F(-0.25), F(0.25), F(0.5))        # u' = -1, v' = 0
+    d = O.equirect_dir(F(-1.125), F(-0.25), F(0.25), F(0.5))        # u' = -1, v' = 0
     assert np.allclose(d, [0, 0, 1], atol=1e-7)
     assert abs(abs(np.arctan2(d[0], -d[2])) - np.pi) < 1e-6
 
@@ -75,7 +73,7 @@ def test_every_pixel_looks_at_its_texel_centre(w, h):
     if w % 4 == 0:                                                  # u' = -1/2 and +1/2 lie on column boundaries
         pw, ph = F(2) / F(w), F(2) / F(h)
         for u, x in ((-0.5, -1.0), (0.5, 1.0)):
-            d = OC.equirect_dir(F(u) - pw / F(2), F(-ph / F(2)), pw, ph)
+            d = O.equirect_dir(F(u) - pw / F(2), F(-ph / F(2)), pw, ph)
             assert np.allclose(d, [x, 0, 0], atol=1e-7), (u, d)
 
 
@@ -120,8 +118,8 @@ def test_rotated_camera_rotates_every_direction():
     w, h, spp = 24, 12, 3
     rays = {}
     for key, r, t in (("plain", None, (0, 0, 0)), ("rotated", rotation(3), (1.5, -2.0, 0.25))):
-        osc = OC.CameraOracleScene(camera_doc(r, t))
-        osc.set_projection(0, OC.EQUIRECTANGULAR)
+        osc = O.OracleScene(camera_doc(r, t))
+        osc.set_projection(0, O.EQUIRECTANGULAR)
         rays[key] = panorama_rays(osc, w, h, spp)
     R = rotation(3).astype(np.float32).astype(np.float64)
     assert np.abs(rays["rotated"][:, 3:] - rays["plain"][:, 3:] @ R.T).max() < 1e-6
@@ -138,8 +136,8 @@ def test_every_ray_lands_in_its_pixels_texel(focus):
     rounded pi/2 is -4.4e-8): there it may come out half a turn off.  Focus or not, every origin is the camera position."""
     w, h, spp = 40, 20, 8
     R, t = rotation(5), (0.5, 1.0, -3.0)
-    osc = OC.CameraOracleScene(camera_doc(R, t, focus))
-    osc.set_projection(0, OC.EQUIRECTANGULAR)
+    osc = O.OracleScene(camera_doc(R, t, focus))
+    osc.set_projection(0, O.EQUIRECTANGULAR)
     rays = panorama_rays(osc, w, h, spp, seed=7)
     assert np.array_equal(rays[:, :3], np.tile(F(t), (len(rays), 1)))
     d = rays[:, 3:].astype(np.float64) @ R.astype(np.float32).astype(np.float64)   # back to camera space
@@ -198,9 +196,9 @@ def test_round_trip_reproduces_the_map():
     of the two); a half-texel shift of the convention would be ~20 x that"""
     h, w, spp = 24, 48, 128
     env = smooth_map(h, w, 21)
-    osc = OC.CameraOracleScene(camera_doc())
+    osc = O.OracleScene(camera_doc())
     osc.set_environment(env)
-    osc.set_projection(0, OC.EQUIRECTANGULAR)
+    osc.set_projection(0, O.EQUIRECTANGULAR)
     a, n, _ = oracle_render(osc, 0, w, h, spp, seed=1)
     b, _, _ = oracle_render(osc, 0, w, h, spp, seed=2)
     err, noise = round_trip_error(a, b, n, env)
@@ -219,8 +217,8 @@ def test_einstein_ring_in_a_panorama():
     doc, pos, fwd, right = ring_scene()
     theta_e = einstein_angle_f64(pos, fwd, right)
     w, h, spp = 512, 256, 4
-    osc = OC.CameraOracleScene(doc)
-    osc.set_projection(0, OC.EQUIRECTANGULAR)
+    osc = O.OracleScene(doc)
+    osc.set_projection(0, O.EQUIRECTANGULAR)
     osc.set_environment(disc_map(fwd))
     dirs = panorama_rays(osc, w, h, spp)[:, 3:].astype(np.float64)
     ang = np.arccos(np.clip((dirs @ fwd) / np.linalg.norm(dirs, axis=1), -1, 1)).reshape(h, w, spp).mean(-1)
@@ -241,21 +239,23 @@ def test_einstein_ring_in_a_panorama():
             assert (ang[lum > 0] <= DISC + 2 * np.pi / 2048 + pixel).all()
 
 
-# ---- the oracle without a projection is oracle_env --------------------------------------------------------------------------
+# ---- PERSPECTIVE is no projection -------------------------------------------------------------------------------------------
 
-def test_camera_oracle_without_a_projection_is_the_env_oracle():
+def test_back_to_perspective_is_no_projection():
+    """a camera set to PERSPECTIVE, then switched to EQUIRECTANGULAR and back, renders bit for bit what the camera of a
+    freshly loaded scene that never had a projection renders"""
     for name, lens, env in (("scene", LENS_SCENE, smooth_map(16, 32, 3)), ("cloud", None, None), ("cornell", None, None)):
         w, h = 48, 27
-        env_osc = OE.load_pair(name, w, h, lenses=lens)[0]
-        osc, _, cam = OC.load_pair(name, w, h, lenses=lens, projection=OC.PERSPECTIVE)
+        fresh, _, cam = load_pair(name, w, h, lenses=lens)
+        osc = load_pair(name, w, h, lenses=lens, projection=O.PERSPECTIVE)[0]
         if env is not None:
-            env_osc.set_environment(env)
+            fresh.set_environment(env)
             osc.set_environment(env)
-        ref = oracle_render(env_osc, cam, w, h, 1, 2, seed=4)[0]
+        ref = oracle_render(fresh, cam, w, h, 1, 2, seed=4)[0]
         assert np.array_equal(oracle_render(osc, cam, w, h, 1, 2, seed=4)[0], ref), name
-        osc.set_projection(cam, OC.EQUIRECTANGULAR)
+        osc.set_projection(cam, O.EQUIRECTANGULAR)
         assert not np.array_equal(oracle_render(osc, cam, w, h, 1, 2, seed=4)[0], ref), name
-        osc.set_projection(cam, OC.PERSPECTIVE)
+        osc.set_projection(cam, O.PERSPECTIVE)
         assert np.array_equal(oracle_render(osc, cam, w, h, 1, 2, seed=4)[0], ref), name
 
 
