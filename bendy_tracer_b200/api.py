@@ -498,12 +498,12 @@ class Tracer:
         """scheduling counters of the pooled kernel for the render call with these arguments (bt_render_pool_stats)"""
         engine = self.engine or Engine.default(0)
         cfg, rc = self.config._c(), config._c()
-        out = (C.c_uint64 * 17)()
+        out = (C.c_uint64 * 21)()
         check(lib.bt_render_pool_stats(engine.handle, scene.handle, camera, C.byref(cfg), C.byref(rc), self.seed, sample_base,
                                        width, height, out))
         keys = ("step_iterations", "step_lanes", "refill_rounds", "step_entries", "scan_passes", "scan_slots", "shade_passes",
                 "shade_slots", "regen_passes", "paths_issued", "paths_retired", "turns", "clk_step", "clk_scan", "clk_shade", "clk_regen",
-                "clk_total")
+                "clk_total", "refresh_iterations", "refresh_mixed_iterations", "refresh_lanes_grid", "refresh_lanes_outside")
         d = dict(zip(keys, [int(v) for v in out]))
         d["lanes_per_step"] = d["step_lanes"] / max(d["step_iterations"], 1)
         d["lanes_per_scan"] = d["scan_slots"] / max(d["scan_passes"], 1)

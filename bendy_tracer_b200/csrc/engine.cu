@@ -1005,11 +1005,11 @@ int bt_render_stats(bt_engine* engine, bt_scene* scene, uint64_t camera_ref, con
 
 int bt_render_pool_stats(bt_engine* engine, bt_scene* scene, uint64_t camera_ref, const bt_config* config,
                          const bt_render_config* rc, uint64_t seed, uint64_t sample_base, uint32_t width, uint32_t height,
-                         uint64_t stats_out[17]) {
+                         uint64_t stats_out[21]) {
     if (!engine || !scene || !config || !rc || !stats_out) return fail(BT_ERR_INVALID_ARG, "NULL argument");
     GUARD_BEGIN
     if (int b = bind_scene(engine, scene)) return b;
-    for (int i = 0; i < 17; ++i) stats_out[i] = 0;
+    for (int i = 0; i < 21; ++i) stats_out[i] = 0;
     if (rc->samples == 0) return BT_OK;
     CK(cudaSetDevice(engine->device));
     SceneDev* sdev = 0;
@@ -1029,10 +1029,10 @@ int bt_render_pool_stats(bt_engine* engine, bt_scene* scene, uint64_t camera_ref
     cudaError_t ce = use_exact(engine, scene) ? launch_render_exact(p, engine->stream, &engine->launches) : launch_render_fast(p, engine->stream, &engine->launches);
     if (ce == cudaErrorNotSupported) return fail(BT_ERR_UNSUPPORTED, "scheduling counters exist for the content-specialised pooled kernels only");
     CK(ce);
-    unsigned long long host[17];
+    unsigned long long host[21];
     CK(cudaMemcpyAsync(host, p.stats, sizeof host, cudaMemcpyDeviceToHost, engine->stream));
     CK(cudaStreamSynchronize(engine->stream));
-    for (int i = 0; i < 17; ++i) stats_out[i] = host[i];
+    for (int i = 0; i < 21; ++i) stats_out[i] = host[i];
     return BT_OK;
     GUARD_END
 }

@@ -119,34 +119,45 @@ BT_DEV void flight_reset(Flight& f) {
 // (SceneHeader::dist_*, built by scene.cpp: build_dist_grid) and the exact distance of its scene-spanning spheres.
 // One byte load.  It is split in two so that the load is ISSUED before the RK4 arithmetic of the step that needs it
 // and its value first TOUCHED after (grid_bound_finish): L2 latency then hides under ~150 instructions.
+// One straight sequence for every refreshing lane: the byte load is predicated on "inside the box", the outside bound is
+// computed by all and selected away inside -- a warp whose refreshing lanes sit on both sides of the box faces runs the
+// block once, not an in-box and an out-of-box path one after the other.  The outside part is skipped, warp-uniformly, when
+// no lane running the block is outside.  The far spheres come from the call's constants (SceneHeader::far_c / far_k),
+// unrolled on the uniform n_far.
 struct GridFetch {
     uint32_t raw;   // the cell's byte (inside the box)
     float other;    // min(outside-the-box bound or +inf, the scene-spanning spheres' exact bounds)
+    bool inside;
 };
-BT_DEV GridFetch grid_bound_fetch(const RenderParams& p, const float4* prims, P3 px) {
+BT_DEV float far_sphere_bound(const SceneHeader& s, int i, V3 x) {
+    const float4 q0 = make_float4(s.far_c[i][0], s.far_c[i][1], s.far_c[i][2], s.far_c[i][3]);
+    const float4 q1 = make_float4(0.0f, 0.0f, s.far_k[i], 0.0f);
+    const V3 oc = x - v3(q0);
+    return sphere_free_bound(q0, q1, fmaf(oc.z, oc.z, fmaf(oc.y, oc.y, oc.x * oc.x)));
+}
+BT_DEV GridFetch grid_bound_fetch(const RenderParams& p, P3 px) {
     const SceneHeader& s = p.scene;
     // cell index: a negative coordinate converts to a negative int, i.e. a huge unsigned one
-    const float2 cxy = __fmul2_rn(__fadd2_rn(px.xy, make_float2(-s.dist_lo[0], -s.dist_lo[1])), f2(s.dist_inv_cell));
+    const float2 cxy = __ffma2_rn(px.xy, f2(s.dist_inv_cell), make_float2(s.dist_off[0], s.dist_off[1]));
     const uint32_t ix = (uint32_t)__float2int_rd(cxy.x), iy = (uint32_t)__float2int_rd(cxy.y),
-                   iz = (uint32_t)__float2int_rd(__fmul_rn(__fsub_rn(px.z, s.dist_lo[2]), s.dist_inv_cell));
-    const V3 x = v3(px);
+                   iz = (uint32_t)__float2int_rd(__fmaf_rn(px.z, s.dist_inv_cell, s.dist_off[2]));
+    const bool inside = ix < s.dist_nx && iy < s.dist_ny && iz < s.dist_nz;
     GridFetch g;
+    g.inside = inside;
     g.raw = 0xffffu;  // (x q: beyond every stored value -- the box does not bound this point, `other` does)
+    if (inside) g.raw = __ldg(p.dist + ((iz * s.dist_ny + iy) * s.dist_nx + ix));
     g.other = __int_as_float(0x7f800000);
-    if (ix < s.dist_nx && iy < s.dist_ny && iz < s.dist_nz) {
-        g.raw = __ldg(p.dist + ((iz * s.dist_ny + iy) * s.dist_nx + ix));
-    } else {  // outside the box: every gridded primitive lies dist_pad inside its faces; the scene-spanning spheres exactly
+    // (every lane that runs this block takes part in the vote, so an outside lane always sees it true)
+    if (__any_sync(__activemask(), !inside)) {
+        // outside the box: every gridded primitive lies dist_pad inside its faces; the scene-spanning spheres exactly
+        const V3 x = v3(px);
         const float dx = fmaxf(fmaxf(s.dist_lo[0] - x.x, x.x - s.dist_hi[0]), 0.0f);
         const float dy = fmaxf(fmaxf(s.dist_lo[1] - x.y, x.y - s.dist_hi[1]), 0.0f);
         const float dz = fmaxf(fmaxf(s.dist_lo[2] - x.z, x.z - s.dist_hi[2]), 0.0f);
-        g.other = (sqrt_approx(fmaf(dz, dz, fmaf(dy, dy, dx * dx))) + s.dist_pad) * 0.999f - 1e-3f;
-#pragma unroll 1
-        for (uint32_t i = 0; i < s.n_far; ++i) {  // (0 .. 2, uniform)
-            const float4* q = prims + s.far_prim[i] * PRIM_STRIDE;
-            const float4 q0 = q[0], q1 = q[1];
-            const V3 oc = x - v3(q0);
-            g.other = fminf(g.other, sphere_free_bound(q0, q1, fmaf(oc.z, oc.z, fmaf(oc.y, oc.y, oc.x * oc.x))));
-        }
+        float other = (sqrt_approx(fmaf(dz, dz, fmaf(dy, dy, dx * dx))) + s.dist_pad) * 0.999f - 1e-3f;
+        if (s.n_far > 0) other = fminf(other, far_sphere_bound(s, 0, x));
+        if (s.n_far > 1) other = fminf(other, far_sphere_bound(s, 1, x));
+        if (!inside) g.other = other;
     }
     return g;
 }
@@ -161,8 +172,11 @@ BT_DEV float grid_bound_finish(const RenderParams& p, const GridFetch& g, float 
 // last intersection pass: its distance is evaluated afresh at the chord's start, so a ray that flies
 // along a large surface (the r = 100 ground sphere, a unit or three below most of every path) keeps its
 // free distance instead of spending it after a few steps (C3: 23.7 -> 12.8 intersection passes per path, cloud + lens 28.6 -> 18.8).
+// `refreshed` (the pooled kernel's counters only): 0 no grid refresh in this step, 1 from a cell of the grid, 2 outside its box.
 template <bool EXACT, int C, class L>
-BT_DEV int geodesic_step(const RenderParams& p, const L& lens, const float4* prims, P3& x, P3& v, Flight& f, float tmax) {
+BT_DEV int geodesic_step(const RenderParams& p, const L& lens, const float4* prims, P3& x, P3& v, Flight& f, float tmax,
+                         int* refreshed = nullptr) {
+    if (refreshed) *refreshed = 0;
     float rmin;
     bool captured, far;
     D0Cache<L> cache;
@@ -176,12 +190,14 @@ BT_DEV int geodesic_step(const RenderParams& p, const L& lens, const float4* pri
     GridFetch gf;
     gf.raw = 0;
     gf.other = 0.0f;
+    gf.inside = false;
     // Grid mode: the bound decays with the distance flown (f.free) and is re-read from the grid only when the coming chord
     // (about as long as the last one, f.rest) could outrun it -- a byte gather by all 32 lanes at every step is 32 L1
     // wavefronts per warp instruction and made the step L1-bound (C3: -6 %); a quarter of the lanes is not.
     const bool grid = p.scene.lens_skip == 3, refresh = grid && free <= 1.4f * f.rest;
     if (grid) {
-        if (refresh) gf = grid_bound_fetch(p, prims, f.xp);
+        if (refresh) gf = grid_bound_fetch(p, f.xp);
+        if (refreshed && refresh) *refreshed = gf.inside ? 1 : 2;
     } else if ((C & CT_SPHERES) && f.near >= 0) {
         const float4* q = prims + f.near * PRIM_STRIDE;
         const float4 q0 = q[0], q1 = q[1];

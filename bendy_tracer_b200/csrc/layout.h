@@ -106,11 +106,19 @@ struct SceneHeader {
     // distance from ANY point of the cell to the surface of ANY primitive, already reduced by the rounding margins of the hit
     // tests.  The box spans every primitive but the `n_far` scene-spanning spheres listed in far_prim, with dist_pad to spare:
     // outside it the bound is min(distance to the box + dist_pad, exact distance to those spheres).
+    // A point's cell is floor(fma(x, dist_inv_cell, dist_off)), dist_off = -dist_lo * dist_inv_cell (build_dist_grid checks
+    // that this bins every point of the box within the cells' padding).  far_c / far_k copy the q0 = (c.xyz, r) and q1.z
+    // (margin coefficient) of the far_prim records, so that the stepper evaluates those spheres from the call's constants;
+    // build_dist_grid rewrites them whenever it re-plans the grid (flatten, and every commit of a lensed grid scene).
+    float dist_inv_cell;
+    float dist_off[3];               // (8-byte aligned in the parameter block: the x, y pair is one LDC.64)
     float dist_lo[3], dist_hi[3];
-    float dist_cell, dist_inv_cell, dist_q, dist_pad;
+    float dist_cell, dist_q, dist_pad;
     uint32_t dist_nx, dist_ny, dist_nz;
     uint32_t n_far;
     int32_t far_prim[2];
+    float far_c[2][4];
+    float far_k[2];
 };
 
 enum { PROJ_PERSPECTIVE = 0, PROJ_EQUIRECTANGULAR = 1 };  // BT_PROJECTION_* (bt_scene_set_camera_projection)

@@ -125,7 +125,9 @@ BT_DEV void unpack_hit(uint32_t w, Hit& h) {
 
 // PSTATS: scheduling counters (bt_render_pool_stats; never timed): p.stats[0..11] = STEP iterations, flying lanes summed
 // over them, refill rounds, STEP entries, SCAN passes, slots scanned, SHADE passes, slots shaded, REGEN passes,
-// paths issued, paths retired, turns; [12..16] = SM clocks the warps spent in STEP, SCAN, SHADE, REGEN and in the kernel
+// paths issued, paths retired, turns; [12..16] = SM clocks the warps spent in STEP, SCAN, SHADE, REGEN and in the kernel;
+// [17..20] = free-distance grid refreshes: STEP iterations in which any lane refreshed, those in which lanes inside and
+// outside the grid's box both did, lanes refreshed from a cell of the grid, lanes refreshed outside its box
 template <bool LENS, bool EXACT, int NL, int C, bool PSTATS = false, bool BVH = false>
 BT_DEV void render_pool_body(const RenderParams& p) {
     static_assert(!(BVH && LENS), "the pooled traversal serves flat fields (a lensed BVH scene renders through render_body)");
@@ -166,7 +168,7 @@ BT_DEV void render_pool_body(const RenderParams& p) {
     uint32_t n_node = 0, n_leaf = 0;  // BVH: traversals at an inner node / holding a leaf (n_pend stays 0)
     bool regen_futile = false;
     uint32_t turn = 0, w0 = 0;  // w0: the pool row the slot lists start at (rotates)
-    uint32_t ps[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};  // PSTATS only (warp-uniform)
+    uint32_t ps[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};  // PSTATS only (warp-uniform)
     long long pc[5] = {0, 0, 0, 0, 0}, pc_t0 = 0;            // PSTATS only: SM clocks in STEP / SCAN / SHADE / REGEN, and in all
     if (PSTATS) pc_t0 = clock64();
 
@@ -246,7 +248,17 @@ BT_DEV void render_pool_body(const RenderParams& p) {
                     ++ps[0];
                     ps[1] += __popc(__ballot_sync(0xffffffffu, slot >= 0 && fs == FL_FLY));
                 }
-                if (slot >= 0 && fs == FL_FLY) fs = geodesic_step<EXACT, C>(p, lens, sc.prims, x, v, f, p.clip_max);
+                if (PSTATS) {
+                    int rf = 0;
+                    if (slot >= 0 && fs == FL_FLY) fs = geodesic_step<EXACT, C>(p, lens, sc.prims, x, v, f, p.clip_max, &rf);
+                    const uint32_t n_in = __popc(__ballot_sync(0xffffffffu, rf == 1)), n_out = __popc(__ballot_sync(0xffffffffu, rf == 2));
+                    ps[12] += (n_in + n_out) != 0;
+                    ps[13] += n_in != 0 && n_out != 0;
+                    ps[14] += n_in;
+                    ps[15] += n_out;
+                } else if (slot >= 0 && fs == FL_FLY) {
+                    fs = geodesic_step<EXACT, C>(p, lens, sc.prims, x, v, f, p.clip_max);
+                }
             }
             // park the flights still flying
             {
@@ -650,6 +662,7 @@ BT_DEV void render_pool_body(const RenderParams& p) {
         if (lane == 0) {
             for (int i = 0; i < 12; ++i) atomicAdd(p.stats + i, (unsigned long long)ps[i]);
             for (int i = 0; i < 5; ++i) atomicAdd(p.stats + 12 + i, (unsigned long long)pc[i]);
+            for (int i = 0; i < 4; ++i) atomicAdd(p.stats + 17 + i, (unsigned long long)ps[12 + i]);
         }
     }
 }

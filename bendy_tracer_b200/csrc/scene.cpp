@@ -1283,6 +1283,25 @@ bool build_dist_grid(const std::vector<float4>& prims, const std::vector<Bounds>
     const float q = 0.5f * cell;
     // a point is binned with float arithmetic and may land one ulp into the neighbouring cell: the half diagonal is padded
     const double half_diag = 0.5 * std::sqrt(3.0) * (double)cell * 1.01 + 1e-5;
+    // The stepper bins with fma(x, 1 / cell, -lo / cell): rounded 1 / cell, rounded offset and the rounded sum put a point of
+    // the box at most (|x| / cell + |lo| / cell + index) * 2^-23 cells off its true cell coordinate along each axis.  The
+    // padding above covers a point 0.005 cells outside its cell (sqrt(3) * 0.005 < 0.01 * 0.5 * sqrt(3)); a box that far
+    // from the origin, measured in cells, keeps the per-flight scheme.
+    const float inv_cell = 1.0f / cell;
+    float off[3];
+    for (int k = 0; k < 3; ++k) {
+        off[k] = -box.lo[k] * inv_cell;
+        const double reach = std::max(std::fabs((double)box.lo[k]), std::fabs((double)box.lo[k] + (double)dims[k] * cell)) / cell;
+        if ((2.0 * reach + dims[k] + 2.0) * std::ldexp(1.0, -23) > 0.005) return false;
+    }
+    for (uint32_t i = 0; i < h.n_far; ++i) {  // the far spheres' records, as the stepper reads them (sphere_free_bound)
+        const float4* rec = &prims[(size_t)h.far_prim[i] * PRIM_STRIDE];
+        h.far_c[i][0] = rec[0].x;
+        h.far_c[i][1] = rec[0].y;
+        h.far_c[i][2] = rec[0].z;
+        h.far_c[i][3] = rec[0].w;
+        h.far_k[i] = rec[1].z;
+    }
     // The cells are normally filled ON THE DEVICE (engine.cu: dist_grid_kernel, the same arithmetic in the same order, one thread
     // per cell: a 2M-cell grid takes 65 - 140 ms here and well under a millisecond there); BT_DIST_GRID_HOST=1 fills them here.
     out->clear();
@@ -1319,9 +1338,10 @@ bool build_dist_grid(const std::vector<float4>& prims, const std::vector<Bounds>
     for (int k = 0; k < 3; ++k) {
         h.dist_lo[k] = box.lo[k];
         h.dist_hi[k] = box.lo[k] + (float)dims[k] * cell;
+        h.dist_off[k] = off[k];
     }
     h.dist_cell = cell;
-    h.dist_inv_cell = 1.0f / cell;
+    h.dist_inv_cell = inv_cell;
     h.dist_q = q;
     h.dist_pad = pad;
     h.dist_nx = dims[0];

@@ -260,13 +260,15 @@ int bt_render_stats(bt_engine* engine, bt_scene* scene, uint64_t camera_ref, con
 /* Scheduling counters of the pooled render kernel for the same call (an instrumented copy, never timed):
  * stats_out = {STEP iterations, flying lanes summed over them, refill rounds, STEP entries, SCAN passes,
  * slots scanned, SHADE passes, slots shaded, REGEN passes, paths issued, paths retired, turns, SM clocks the
- * warps spent in STEP, SCAN, SHADE, REGEN, SM clocks of the warps' whole lives} summed over all warps -- lanes
+ * warps spent in STEP, SCAN, SHADE, REGEN, SM clocks of the warps' whole lives, STEP iterations in which a lane
+ * refreshed its free distance from the lensed grid, those in which lanes inside and outside the grid's box both did,
+ * lanes refreshed from a cell of the grid, lanes refreshed outside its box} summed over all warps -- lanes
  * per pass = slots / passes.  BT_ERR_UNSUPPORTED when no content-specialised pooled kernel renders the
  * call: pool_w = 0, a BVH scene, max bounces above 254, more than 126 primitives, or a scene or output
  * that only a generic kernel serves. */
 int bt_render_pool_stats(bt_engine* engine, bt_scene* scene, uint64_t camera_ref, const bt_config* config,
                          const bt_render_config* render_config, uint64_t seed, uint64_t sample_base,
-                         uint32_t width, uint32_t height, uint64_t stats_out[17]);
+                         uint32_t width, uint32_t height, uint64_t stats_out[21]);
 
 /* Buffer::preview, reference src/tracer/buffer.rs:117-138 (+ ColorSpace::convert_linear :19-30,
  * linear_to_srgb / f32_to_u8 src/color.rs:14-24).  rgba8 lives where rgba32f lives. */

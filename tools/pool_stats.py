@@ -39,3 +39,8 @@ print("pool:", {k: (round(v, 2) if isinstance(v, float) else v) for k, v in ps.i
 print(f"per path: step iterations x32 / rk4 steps = {ps['step_iterations'] * 32 / max(st['rk4_steps'], 1):.3f}, "
       f"refill rounds per step iteration = {ps['refill_rounds'] / max(ps['step_iterations'], 1):.3f}, "
       f"step iterations per STEP entry = {ps['step_iterations'] / max(ps['step_entries'], 1):.1f}")
+n_ref = ps["refresh_lanes_grid"] + ps["refresh_lanes_outside"]
+print(f"free-distance refreshes: STEP iterations with one {ps['refresh_iterations'] / max(ps['step_iterations'], 1):.3f}, "
+      f"with lanes inside and outside the box {ps['refresh_mixed_iterations'] / max(ps['refresh_iterations'], 1):.3f} of those, "
+      f"lanes per such iteration {n_ref / max(ps['refresh_iterations'], 1):.2f}, outside the box {ps['refresh_lanes_outside'] / max(n_ref, 1):.3f} of the lanes, "
+      f"per RK4 step {n_ref / max(st['rk4_steps'], 1):.3f}")
